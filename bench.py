@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the B200 CG path (contract: see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--variant pr] [--grid 256] [--dim 3] [--iters 200]
+                    [--variant pr] [--grid 256] [--dim 3] [--iters 200] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3], the one the metric is quoted on): 3-D Poisson 7-point,
 256^3 grid (16.8 M unknowns), Jacobi-preconditioned, x_true = 1/sqrt(n), b = A x_true,
@@ -116,6 +116,20 @@ def pinned(a):
     import torch
     t = torch.from_numpy(np.ascontiguousarray(a)).pin_memory()
     return t, t.numpy()
+
+
+DUMP_MAX_ENTRIES = 1 << 22        # 32 MB of float64
+
+
+def dump_outputs(out_dir, x):
+    """--dump-outputs: the solution x of the last timed step as out_dir/x.npy (float64).  Above
+    DUMP_MAX_ENTRIES entries it holds x at the sorted indices
+    np.random.default_rng(0).choice(n, DUMP_MAX_ENTRIES, replace=False): the same entries for
+    the same arguments, so that two builds can be compared output for output."""
+    if x.shape[0] > DUMP_MAX_ENTRIES:
+        x = x[np.sort(np.random.default_rng(0).choice(x.shape[0], DUMP_MAX_ENTRIES, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x.npy"), np.ascontiguousarray(x, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------ reference arm
@@ -335,6 +349,10 @@ def run_ours(args, rank, world, local_rank):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dev_ms, loop_ms, wall_ms = t.tolist()
     value = its * args.steps / (dev_ms / 1e3)
+    if args.dump_outputs:              # before the e2e pass below overwrites x
+        x = sess.fetch(want_hist=False)[0] if world == 1 else sess.gather_x(sess.fetch_local(want_hist=False)[0])
+        if rank == 0:
+            dump_outputs(args.dump_outputs, x)
 
     # ---- e2e through the C-ABI call with host buffers (pinned), copies inside the timing
     e2e = None
@@ -656,12 +674,17 @@ def main():
     ap.add_argument("--tail-grid", type=int, default=64)
     ap.add_argument("--tail-iters", type=int, default=2000)
     ap.add_argument("--tail-reps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the solution x of the last one to DIR/x.npy "
+                         "(float64; a fixed seeded sample above %d entries)" % DUMP_MAX_ENTRIES)
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.steps < 1 or args.warmup < 0:
         ap.error("steps >= 1, warmup >= 0")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "headline"):
+        ap.error("--dump-outputs writes the outputs of the headline workload (--impl ours --config headline)")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

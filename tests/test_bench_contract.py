@@ -1,9 +1,13 @@
 """CPU (-m "not gpu"): the reference arm of bench.py runs without a GPU (it times the oracle port
-on the host cores) -- check the one-JSON-line contract and its keys on a tiny grid."""
+on the host cores) -- check the one-JSON-line contract and its keys on a tiny grid.  GPU: the
+outputs --dump-outputs writes for the timed arm."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -55,3 +59,47 @@ def test_traffic_stamps_match_the_kernel_sources():
     assert bench.read_traffic("no_such_kernel")[0] is None
     # a class's stamp ignores headers its kernel is not compiled from
     assert b.kernel_fingerprint("pr_fused") != b.kernel_fingerprint("csr_sp_pr") != b.kernel_fingerprint()
+
+
+def test_dump_outputs_sample_is_fixed_and_other_arms_refuse_it(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    n = bench.DUMP_MAX_ENTRIES + 1000
+    x = np.arange(n, dtype=np.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), x)
+    sa, sb = np.load(tmp_path / "a" / "x.npy"), np.load(tmp_path / "b" / "x.npy")
+    assert sa.dtype == np.float64 and sa.shape == (bench.DUMP_MAX_ENTRIES,)
+    assert np.array_equal(sa, sb) and np.all(np.diff(sa) > 0)      # same entries, in index order
+    bench.dump_outputs(str(tmp_path / "small"), x[:100])
+    assert np.array_equal(np.load(tmp_path / "small" / "x.npy"), x[:100])
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--grid", "12",
+                          "--dump-outputs", str(tmp_path / "ref")], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode != 0 and out.stdout.strip() == "" and not (tmp_path / "ref").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_solution_of_the_timed_steps(tmp_path):
+    """--dump-outputs writes x of the last timed step: bit for bit what a direct Session run of the
+    same workload returns, whatever --steps is; --steps sets the number of timed solves."""
+    sys.path.insert(0, ROOT)
+    import bench
+    from new_cg_variants_b200 import Session
+    runs = {}
+    for steps in (2, 3):
+        d = tmp_path / f"steps{steps}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--grid", "12", "--iters", "20",
+                              "--steps", str(steps), "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert sorted(os.listdir(d)) == ["x.npy"]
+        runs[steps] = (json.loads(out.stdout), np.load(d / "x.npy"))
+    assert runs[2][0]["steps"] == 2 and runs[3][0]["steps"] == 3
+    assert 2 * runs[3][0]["gpu_launches"] == 3 * runs[2][0]["gpu_launches"]
+    S, b, x0, x_true, dinv = bench.build_problem(12)
+    with Session(S, dinv=dinv) as s:
+        s.load_problem(b, x0, None)
+        s.run("pr", 21, histories=(), path="auto")
+        x = s.fetch(want_hist=False)[0]
+    for _, dumped in runs.values():
+        assert dumped.dtype == np.float64 and np.array_equal(dumped, x)

@@ -1,5 +1,5 @@
-import sys, numpy as np
-sys.path.insert(0, "/root/repo")
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from new_cg_variants_b200 import PoissonStencil, Session
 S = PoissonStencil(256, 256, 256, dim=3); n = S.shape[0]
 b, x0 = S @ (np.ones(n)/np.sqrt(n)), np.zeros(n)

@@ -1,5 +1,5 @@
-import sys, numpy as np
-sys.path.insert(0, "/root/repo")
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from new_cg_variants_b200 import PoissonStencil, Session
 for shape in ((256,256,32),(256,256,16),(256,256,64),(64,64,64)):
     S = PoissonStencil(*shape, dim=3); n = S.shape[0]
