@@ -256,6 +256,29 @@ int cgx_group_begin(cgx_ctx** ctxs, int count, int variant, int max_iter, unsign
                     int path);
 int cgx_group_advance(cgx_ctx** ctxs, int count, int niter);
 
+/* ---- independent solves side by side on one GPU (e.g. the nine variants of one case,
+ *      figure_gen.py:50-60, or one matrix with several right-hand sides).  Runs ctxs[i] as
+ *      cgx_run(ctxs[i], variants[i], max_iters[i], hist_mask, CGX_PATH_PERSISTENT, &infos[i])
+ *      would, except that all entries share one cooperative launch: entry i gets its own CTA
+ *      range, sized by the persistent geometry for a 1/count share of the SMs (so its dot
+ *      products are summed in the order of a solo run with that CTA shape -- its results are
+ *      bitwise those of cgx_run with "pers_threads" / "pers_ctas" set to that shape, not
+ *      necessarily those of a default cgx_run).  Entries never wait for each other; one with a
+ *      smaller max_iter finishes first.  Each context keeps its own operator, preconditioner and
+ *      problem (b, x0, optional x_true), loaded beforehand; results are fetched per context as
+ *      after cgx_run.  The CTA width is common to the batch: the contexts' "pers_threads" when
+ *      set (they must agree), else chosen so that every entry fits; "pers_ctas" and "csr_slab"
+ *      act per entry as in cgx_run.  infos[i].loop_ms is the duration of the SHARED launch.
+ *      Returns CGX_ERR_BREAKDOWN if any entry broke down (infos[i].breakdown_iter tells which).
+ *      CGX_ERR_ARG: count < 1, a NULL pointer, a bad variant or max_iter, a context listed twice.
+ *      CGX_ERR_UNSUPPORTED, before anything is launched: entries on different devices, a rank of
+ *      a partition, mixed operator kinds (CSR / stencil) or preconditioner modes (none / Jacobi
+ *      vector / constant diagonal), a capture, a GV replacement schedule or "gv_manual" set, an
+ *      entry that does not fit its share of the SMs, or a grid that is not co-resident.  After a
+ *      refusal every context still runs normally with cgx_run. */
+int cgx_batch_run(cgx_ctx** ctxs, int count, const int* variants, const int* max_iters,
+                  unsigned hist_mask, cgx_info* infos);
+
 /* ---- single primitives, exposed for the unit tests of SURVEY.md section 7:
  *      y = A v (scipy `A @ v`) and the deterministic fp64 dot (numpy `u @ v`). */
 int cgx_spmv_host(cgx_ctx* ctx, const double* v_host, double* y_host, int64_t n);

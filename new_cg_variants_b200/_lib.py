@@ -87,6 +87,7 @@ PROTOTYPES = {
     "cgx_group_load_problem_host": (C.c_int, [C.POINTER(_P), C.c_int, c_double_p, c_double_p, c_double_p, C.c_int64]),
     "cgx_group_begin": (C.c_int, [C.POINTER(_P), C.c_int, C.c_int, C.c_int, C.c_uint, C.c_int]),
     "cgx_group_advance": (C.c_int, [C.POINTER(_P), C.c_int, C.c_int]),
+    "cgx_batch_run": (C.c_int, [C.POINTER(_P), C.c_int, c_int32_p, c_int32_p, C.c_uint, C.POINTER(CgxInfo)]),
     "cgx_spmv_host": (C.c_int, [_P, c_double_p, c_double_p, C.c_int64]),
     "cgx_dot_host": (C.c_int, [_P, c_double_p, c_double_p, C.c_int64, c_double_p]),
 }

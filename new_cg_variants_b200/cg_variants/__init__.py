@@ -18,6 +18,9 @@ scaling (identity or Jacobi, figure_gen.py:40-44), otherwise ``NotImplementedErr
 Extra keyword arguments understood here (all optional, ignored by the reference):
 ``device=0``, ``path="auto"|"stream"|"persistent"``, ``session=Session`` (reuse an operator
 already resident on the GPU), ``return_info=True`` (adds ``output['_info']``).
+
+``solve_concurrently(methods, A, b, x0, max_iter, ...)`` runs several of these solvers on the same
+problem in one cooperative launch (figure_gen.py:50-60 runs the nine variants one after another).
 """
 from __future__ import annotations
 
@@ -336,9 +339,72 @@ def _make(name, tag, preconditioned, gv=False):
     return f
 
 
+def solve_concurrently(methods, A, b, x0, max_iter, preconditioner=lambda x: x, callbacks=[], **kwargs):
+    """Run several of this module's solvers on the same problem side by side: ONE cooperative launch
+    on one GPU (``session.solve_batch``), each method on a 1/len(methods) share of the SMs.
+
+    ``methods``: distinct functions of this module (e.g. ``experiments.ALL_METHODS``), preconditioned
+    or all un-preconditioned.  Returns ``{method name: output}``, each output with the keys, names and
+    shapes ``method(A, b, x0, max_iter, preconditioner=..., callbacks=..., **kwargs)`` returns.  The
+    histories are bitwise those of a solo persistent-path run with the same CTA shape (not
+    necessarily of a default solo run, whose CTA shape takes all the SMs).
+
+    Only the four standard callbacks and ``print_k`` are served; any other callback, ``w_replace``,
+    ``path=`` or ``session=`` raises ``NotImplementedError`` before the GPU is touched.  One Session
+    per method, closed afterwards (the operator cache of the single-method functions is not used).
+    Extra keyword arguments: ``x_true``, ``device=0``, ``return_info=True``."""
+    from ..session import solve_batch
+    methods = list(methods)
+    for key in ("path", "w_replace", "session"):
+        if key in kwargs:
+            raise NotImplementedError(f"solve_concurrently: `{key}=` is not supported (persistent batch only)")
+    tags = []
+    for m in methods:
+        name = getattr(m, "__name__", "")
+        stem, _, suffix = name.rpartition("_")
+        if globals().get(name) is not m or suffix not in ("cg", "pcg"):
+            raise NotImplementedError(f"solve_concurrently: {name or m!r} is not a GPU solver of this module")
+        tags.append((name, stem, suffix == "pcg"))
+    if len({t[0] for t in tags}) != len(tags):
+        raise ValueError("solve_concurrently: a method is listed twice")
+    dev_hist, ticks, generic = _split_callbacks(list(callbacks))
+    if generic:
+        raise NotImplementedError("solve_concurrently: only the four standard callbacks and print_k run in a batch; "
+                                  f"got {[getattr(cb, '__name__', cb) for cb in generic]}")
+    device = kwargs.pop("device", 0)
+    return_info = kwargs.pop("return_info", False)
+    n = len(b)
+    _ensure_x_true(A, b, kwargs, any("error" in h for h in dev_hist))
+    x_true = kwargs.get("x_true")
+    dinv = probe_preconditioner(preconditioner, n) if any(t[2] for t in tags) else None
+    sessions = []
+    try:
+        for _, _, pre in tags:
+            sessions.append(Session(A, dinv=dinv if pre else None, device=device))
+        res = solve_batch([(s, tag, b, x0, max_iter, x_true) for s, (_, tag, _) in zip(sessions, tags)],
+                          histories=tuple(dev_hist), return_x=False)
+    finally:
+        for s in sessions:
+            s.close()
+    outputs = {}
+    for (name, _, _), (_, hist, info) in zip(tags, res):
+        output = {"name": name, "max_iter": max_iter}
+        for h in dev_hist:
+            output[h] = hist[h]
+        for cb in ticks:
+            try:
+                cb(output=output, k=max_iter - 1, max_iter=max_iter)
+            except Exception:
+                pass
+        if return_info:
+            output["_info"] = info
+        outputs[name] = output
+    return outputs
+
+
 _TAGS = [("hs", "hs"), ("cg", "cg"), ("gv", "gv"), ("pr", "pr"), ("m", "m"), ("pipe_pr", "pipe_pr"),
          ("pipe_p", "pipe_p"), ("pipe_pr_m", "pipe_pr_m"), ("pipe_p_m", "pipe_p_m")]
-__all__ = ["probe_preconditioner", "clear_cache"]
+__all__ = ["probe_preconditioner", "clear_cache", "solve_concurrently"]
 for _stem, _tag in _TAGS:
     for _suffix, _pre in (("_pcg", True), ("_cg", False)):
         _fname = _stem + _suffix

@@ -161,7 +161,7 @@ extern "C" int cgx_ctx_destroy(cgx_ctx* c) {
   dist_release(c);
   free_state(c); free_problem(c); free_op(c);
   cudaFree(c->d_dinv); cudaFree(c->d_sc); cudaFree(c->d_partials); cudaFree(c->d_ticket);
-  cudaFree(c->d_ppart); cudaFree(c->d_pbar); cudaFree(c->d_pout); cudaFree(c->d_prank); cudaFree(c->d_dbg_t); cudaFree(c->d_tma_err);
+  cudaFree(c->d_ppart); cudaFree(c->d_pbar); cudaFree(c->d_pout); cudaFree(c->d_prank); cudaFree(c->d_pbatch); cudaFree(c->d_dbg_t); cudaFree(c->d_tma_err);
   for (auto& e : c->ev) cudaEventDestroy(e);
   for (auto& e : c->prof_events) cudaEventDestroy(e);
   cudaStreamDestroy(c->own_stream);
@@ -1122,6 +1122,163 @@ extern "C" int cgx_group_load_problem_host(cgx_ctx** cs, int count, const double
   group_share_stream(cs, count, false);
   if (!rc && off != n_total) return fail(CGX_ERR_ARG, "cgx_group_load_problem_host: slabs cover %lld rows, n = %lld",
                                          (long long)off, (long long)n_total);
+  return rc;
+}
+
+// ---------------------------------------------------------------------------------------
+// batch: independent single-GPU solves in ONE cooperative launch (include/cgx.h cgx_batch_run)
+// ---------------------------------------------------------------------------------------
+static int pers_batch(cgx_ctx** cs, int count, const int* variants, const PersGeom* G, const int* k1, bool launch) {
+  const cgx_ctx* c = cs[0];
+  if (c->op_kind == 1) {
+    if (c->pm == 2) return cgx_pers_batch_csr_pm2(cs, count, variants, G, k1, launch);
+    if (c->pm == 1) return cgx_pers_batch_csr_pm1(cs, count, variants, G, k1, launch);
+    return cgx_pers_batch_csr_pm0(cs, count, variants, G, k1, launch);
+  }
+  if (c->pm == 2) return cgx_pers_batch_sten_pm2(cs, count, variants, G, k1, launch);
+  if (c->pm == 1) return cgx_pers_batch_sten_pm1(cs, count, variants, G, k1, launch);
+  return cgx_pers_batch_sten_pm0(cs, count, variants, G, k1, launch);
+}
+
+// The CTA width common to the batch: the contexts' "pers_threads" when set (they must agree);
+// otherwise, among the widths pers_geometry would pick for the entries on their own, the one with
+// which every entry fits, most CSR entries keep their matrix rows in shared memory, and CTAs are widest.
+static int batch_geometry(cgx_ctx** cs, int count, const int* variants, std::vector<PersGeom>& G) {
+  int T = 0;
+  for (int i = 0; i < count; ++i) {
+    if (!cs[i]->pers_threads) continue;
+    if (T && cs[i]->pers_threads != T)
+      return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: the entries' pers_threads differ (%d, %d); one CTA width per launch",
+                  T, cs[i]->pers_threads);
+    T = cs[i]->pers_threads;
+  }
+  std::vector<int> cand;
+  if (T) cand.push_back(T);
+  else
+    for (int i = 0; i < count; ++i) cand.push_back(pers_geometry(cs[i], variants[i], count).T);
+  int best[3] = {-1, -1, -1};
+  std::vector<PersGeom> H(count);
+  for (int t : cand) {
+    int ok = 0, slabs = 0;
+    for (int i = 0; i < count; ++i) {
+      H[i] = pers_geometry_T(cs[i], variants[i], count, t);
+      ok += H[i].ok ? 1 : 0;
+      slabs += H[i].slab_cap > 0 ? 1 : 0;
+    }
+    const int score[3] = {ok == count ? 1 : 0, slabs, H[0].T};
+    if (std::lexicographical_compare(best, best + 3, score, score + 3)) {
+      std::copy(score, score + 3, best);
+      G = H;
+    }
+  }
+  for (int i = 0; i < count; ++i)
+    if (!G[i].ok)
+      return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d (%lld rows x %d resident vectors) does not fit the shared "
+                  "memory of its 1/%d share of the SMs (%zu B per CTA)", i, (long long)cs[i]->n, G[i].nslot, count, G[i].smem);
+  return CGX_OK;
+}
+
+static int batch_run(cgx_ctx** cs, int count, const int* variants, const int* max_iters, unsigned hist_mask, cgx_info* infos) {
+  // ---- refusals: nothing has been enqueued yet -------------------------------------------
+  for (int i = 0; i < count; ++i) {
+    const cgx_ctx* c = cs[i];
+    if (c->op_kind == 0 || !c->problem_loaded) return fail(CGX_ERR_ARG, "cgx_batch_run: entry %d has no operator or problem", i);
+    for (int j = 0; j < i; ++j)
+      if (cs[j] == c) return fail(CGX_ERR_ARG, "cgx_batch_run: entries %d and %d are the same context", j, i);
+    if (c->device != cs[0]->device) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entries on different devices");
+    if (c->dist.world > 1) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d is a rank of a partition", i);
+    if (c->op_kind != cs[0]->op_kind) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: CSR and stencil operators mixed");
+    if (c->pm != cs[0]->pm) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: preconditioner modes mixed (%d, %d)", cs[0]->pm, c->pm);
+    if (c->capture_req) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d has a capture set (stream path only)", i);
+    if (std::any_of(c->gv_replace.begin(), c->gv_replace.end(), [](uint8_t f) { return f != 0; }))
+      return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d has a GV replacement schedule (stream path only)", i);
+    if (c->gv_manual) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d has gv_manual set (stream path only)", i);
+  }
+  CU(cudaSetDevice(cs[0]->device));
+  std::vector<PersGeom> G(count);
+  int rc = batch_geometry(cs, count, variants, G);
+  if (rc) return rc;
+  // entries with max_iter == 1 have no loop to run (as cgx_run: no launch)
+  std::vector<cgx_ctx*> lc;
+  std::vector<int> lv, lk;
+  std::vector<PersGeom> lg;
+  for (int i = 0; i < count; ++i)
+    if (max_iters[i] > 1) { lc.push_back(cs[i]); lv.push_back(variants[i]); lk.push_back(max_iters[i] - 1); lg.push_back(G[i]); }
+  if (!lc.empty()) {
+    rc = pers_batch(lc.data(), (int)lc.size(), lv.data(), lg.data(), lk.data(), false);
+    if (rc) return rc;
+  }
+
+  // ---- initial state (k = 0) of every entry, on the shared stream ------------------------
+  for (int i = 0; i < count; ++i) {
+    cgx_ctx* c = cs[i];
+    rc = begin_prepare(c, variants[i], max_iters[i], hist_mask, CGX_PATH_PERSISTENT, count);
+    if (rc) return rc;
+    const i64 l0 = c->launches;
+    Steps steps;
+    build_init_steps(c, variants[i], variant_info(variants[i], c->d_dinv != nullptr), steps);
+    CU(cudaEventRecord(c->ev[0], c->stream));
+    for (auto& st : steps) st();
+    cgx_fused_push_initial_halo(c);
+    c->cur_k = 0;
+    if (c->hist_mask) {
+      for (int s = core_stages(c); s < iter_stage_count(c); ++s) {
+        Args g = make_args(c);
+        g.k = 0;
+        iter_stage(c, s, g);
+      }
+    }
+    CU(cudaEventRecord(c->ev[1], c->stream));
+    rc = begin_finish(c, l0);
+    if (rc) return rc;
+    rc = check_device_flags(c, "cgx_batch_run");
+    if (rc) return rc;
+  }
+
+  // ---- the iterations of every entry: one launch -----------------------------------------
+  std::vector<i64> l0(count);
+  for (int i = 0; i < count; ++i) {
+    l0[i] = cs[i]->launches;
+    CU(cudaEventRecord(cs[i]->ev[1], cs[i]->stream));
+  }
+  if (!lc.empty()) {
+    rc = pers_batch(lc.data(), (int)lc.size(), lv.data(), lg.data(), lk.data(), true);
+    if (rc) return rc;
+  }
+  for (int i = 0; i < count; ++i) CU(cudaEventRecord(cs[i]->ev[2], cs[i]->stream));
+  CU(cudaStreamSynchronize(cs[0]->stream));
+  CU(cudaGetLastError());
+  bool broke = false;
+  for (int i = 0; i < count; ++i) {
+    cgx_ctx* c = cs[i];
+    float ms1 = 0.f;
+    CU(cudaEventElapsedTime(&ms1, c->ev[1], c->ev[2]));
+    c->loop_ms = ms1;
+    rc = check_device_flags(c, "cgx_batch_run");
+    if (rc) return rc;
+    if (max_iters[i] > 1) { rc = pers_collect(c); if (rc) return rc; }
+    c->launches_run += c->launches - l0[i];
+    c->cur_k = c->max_iter - 1;
+    rc = cgx_get_info(c, &infos[i]);
+    if (rc) return rc;
+    broke = broke || infos[i].breakdown_iter >= 0;
+  }
+  return broke ? CGX_ERR_BREAKDOWN : CGX_OK;
+}
+
+extern "C" int cgx_batch_run(cgx_ctx** cs, int count, const int* variants, const int* max_iters, unsigned hist_mask,
+                             cgx_info* infos) {
+  if (!cs || count < 1 || !variants || !max_iters || !infos) return fail(CGX_ERR_ARG, "cgx_batch_run: bad arguments");
+  for (int i = 0; i < count; ++i) {
+    if (!cs[i]) return fail(CGX_ERR_ARG, "cgx_batch_run: ctxs[%d] is NULL", i);
+    if (variants[i] < 0 || variants[i] >= CGX_NUM_VARIANTS) return fail(CGX_ERR_ARG, "cgx_batch_run: unknown variant %d", variants[i]);
+    if (max_iters[i] < 1) return fail(CGX_ERR_ARG, "cgx_batch_run: max_iter must be >= 1 (entry %d)", i);
+  }
+  // every entry on the first context's stream, as the ranks of a group (group_share_stream)
+  for (int i = 1; i < count; ++i)
+    if (cs[i]->device == cs[0]->device) cs[i]->stream = cs[0]->own_stream;
+  const int rc = batch_run(cs, count, variants, max_iters, hist_mask, infos);
+  for (int i = 1; i < count; ++i) cs[i]->stream = cs[i]->own_stream;
   return rc;
 }
 

@@ -146,6 +146,8 @@ struct cgx_ctx {
   u64* d_pbar = nullptr;                   // sync-point counter
   PersOut* d_pout = nullptr;
   void* d_prank = nullptr;                 // PersRank<Op>[kMaxWorld] (rank 0 of a group holds all)
+  void* d_pbatch = nullptr;                // PersEntry<Op>[] of the last cgx_batch_run this context led
+  size_t pbatch_bytes = 0;
   double* d_exp[2][2] = {};                // exported SpMV inputs [parity][rhs]
   int pers_threshold = 1 << 19;            // AUTO: rows below which the persistent kernel runs
   int pers_threads = 0, pers_ctas = 0;     // 0 = choose (options "pers_threads", "pers_ctas")
@@ -277,3 +279,7 @@ struct PersGeom { int T, nb, R, nslot, slab_cap; unsigned vmask; size_t smem; bo
 #define CGX_PERS_DECL(name) int name(cgx_ctx** cs, int count, const PersGeom& G, int k0, int k1)
 CGX_PERS_DECL(cgx_pers_launch_csr_pm0); CGX_PERS_DECL(cgx_pers_launch_csr_pm1); CGX_PERS_DECL(cgx_pers_launch_csr_pm2);
 CGX_PERS_DECL(cgx_pers_launch_sten_pm0); CGX_PERS_DECL(cgx_pers_launch_sten_pm1); CGX_PERS_DECL(cgx_pers_launch_sten_pm2);
+// batch of independent solves in one cooperative launch (cgx_batch_run); launch = false: co-residency check only
+#define CGX_PERS_BATCH_DECL(name) int name(cgx_ctx** cs, int count, const int* variants, const PersGeom* G, const int* k1, bool launch)
+CGX_PERS_BATCH_DECL(cgx_pers_batch_csr_pm0); CGX_PERS_BATCH_DECL(cgx_pers_batch_csr_pm1); CGX_PERS_BATCH_DECL(cgx_pers_batch_csr_pm2);
+CGX_PERS_BATCH_DECL(cgx_pers_batch_sten_pm0); CGX_PERS_BATCH_DECL(cgx_pers_batch_sten_pm1); CGX_PERS_BATCH_DECL(cgx_pers_batch_sten_pm2);

@@ -191,24 +191,22 @@ __device__ __forceinline__ void pers_row_slab(const CsrSlab&, int, Ld, double (&
 
 struct PersRec { u64 e; int kind; int k; int hist; };      // a published record still to be folded
 
+// The whole solve of one rank, run by CTA `cta` (0 .. L.nb-1) of the rank's CTA range.  The
+// static shared scratch is declared by the calling kernel, so that a kernel that can run several
+// variants (persistent_batch_kernel) holds one copy of it, not one per inlined body:
+// sh[kPersRed * 32], sh_acc[kPersRed], gg (the rank's global-memory Args), sh_last.
 template <class Op, int VAR, int PM>
-__global__ void __launch_bounds__(512) persistent_kernel(const PersRank<Op>* __restrict__ ranks,
-                                                          const PersLaunch L) {
+__device__ __forceinline__ void persistent_body(const PersRank<Op>& pr, const PersLaunch& L, const int cta,
+                                                double* sh, double* sh_acc, Args& gg, int& sh_last) {
   using P = PersPlan<VAR>;
   constexpr int EW = P::EW, SP = P::SP;
   constexpr bool MEUR = P::MEUR;
   constexpr int NRE = EwTraits<EW>::NR, NRS = SpTraits<SP>::NR, NV = SpTraits<SP>::NV;
   constexpr bool SL = Op::kSlab;
   extern __shared__ __align__(16) double smem[];               // [nslot][R*T]
-  __shared__ double sh[kPersRed * 32];
-  __shared__ double sh_acc[kPersRed];
-  __shared__ Args gg;                                          // this rank's global-memory Args
-  __shared__ int sh_last;
 
   const int T = blockDim.x, tid = threadIdx.x;
   const int nb = L.nb;
-  const int rk = blockIdx.x / nb, cta = blockIdx.x - rk * nb;
-  const PersRank<Op>& pr = ranks[rk];
   const Op A = pr.A;
   if (tid == 0) gg = pr.g;
   __syncthreads();
@@ -606,6 +604,51 @@ __global__ void __launch_bounds__(512) persistent_kernel(const PersRank<Op>* __r
     o->del = s.del; o->gam = s.gam; o->breakdown = s.breakdown;
     pr.out->epoch = epoch;
     for (int c = 0; c < kChan; ++c) pr.out->hepoch[c] = hep[c];
+  }
+}
+
+// One variant; CTA range r*nb .. (r+1)*nb-1 is rank r of ranks[] (one entry on a single GPU).
+template <class Op, int VAR, int PM>
+__global__ void __launch_bounds__(512) persistent_kernel(const PersRank<Op>* __restrict__ ranks,
+                                                          const PersLaunch L) {
+  __shared__ double sh[kPersRed * 32];
+  __shared__ double sh_acc[kPersRed];
+  __shared__ Args gg;
+  __shared__ int sh_last;
+  const int rk = blockIdx.x / L.nb;
+  persistent_body<Op, VAR, PM>(ranks[rk], L, blockIdx.x - rk * L.nb, sh, sh_acc, gg, sh_last);
+}
+
+// A batch of independent single-GPU solves (cgx_batch_run): entry i owns CTAs cta0 .. cta0+L.nb-1
+// and runs its own variant with its own sync counter, partials and PersOut.  Entries never wait
+// for each other; one that has fewer iterations simply finishes first.  The grid is one
+// cooperative launch, so every entry's CTAs are co-resident (separate launches would not be
+// guaranteed to run side by side).  blockDim is common; the dynamic shared memory is the largest
+// entry's.
+template <class Op>
+struct PersEntry {
+  PersRank<Op> r;
+  PersLaunch L;
+  int variant;
+  int cta0;                            // first CTA of the entry (entries in ascending order)
+};
+
+template <class Op, int PM>
+__global__ void __launch_bounds__(512) persistent_batch_kernel(const PersEntry<Op>* __restrict__ entries, int count) {
+  __shared__ double sh[kPersRed * 32];
+  __shared__ double sh_acc[kPersRed];
+  __shared__ Args gg;
+  __shared__ int sh_last;
+  int i = 0;
+  while (i + 1 < count && (int)blockIdx.x >= entries[i + 1].cta0) ++i;
+  const PersEntry<Op>& e = entries[i];
+  const int cta = (int)blockIdx.x - e.cta0;
+  switch (e.variant) {
+#define CGX_PB(V) case V: persistent_body<Op, V, PM>(e.r, e.L, cta, sh, sh_acc, gg, sh_last); break;
+    CGX_PB(CGX_HS) CGX_PB(CGX_CG) CGX_PB(CGX_GV) CGX_PB(CGX_PR) CGX_PB(CGX_M) CGX_PB(CGX_PIPE_PR)
+    CGX_PB(CGX_PIPE_P) CGX_PB(CGX_PIPE_PR_M) CGX_PB(CGX_PIPE_P_M)
+#undef CGX_PB
+    default: break;
   }
 }
 

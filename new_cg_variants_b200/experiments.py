@@ -35,8 +35,13 @@ def setup_problem(A):
     return x_true, b, x0
 
 
-def test_matrix(A, max_iter, title, preconditioner=None, variants=(), data_dir="./data", save=True, **solver_kwargs):
-    """figure_gen.py:21-60.  Returns {method name: output dict}."""
+def test_matrix(A, max_iter, title, preconditioner=None, variants=(), data_dir="./data", save=True, concurrent=False,
+                **solver_kwargs):
+    """figure_gen.py:21-60.  Returns {method name: output dict}.
+
+    ``concurrent=True``: the GPU methods run side by side in one launch (cg_variants.solve_concurrently;
+    bitwise equal to solo runs with the same CTA shape, not to default solo runs); ``exact_pcg``, if listed,
+    is still the reference's own call.  The files written are the same."""
     N = A.get_shape()[0] if hasattr(A, "get_shape") else A.shape[0]
     x_true, b, x0 = setup_problem(A)
     callbacks = [_cb.error_A_norm, _cb.residual_2_norm, _cb.error_2_norm, _cb.updated_residual_2_norm]
@@ -50,8 +55,16 @@ def test_matrix(A, max_iter, title, preconditioner=None, variants=(), data_dir="
     if save:
         os.makedirs(out_dir, exist_ok=True)
     trials = {}
+    batch = {}
+    if concurrent:
+        gpu = [m for m in variants if m.__name__ != "exact_pcg"]
+        if gpu:
+            batch = _cg.solve_concurrently(gpu, A, b, x0, max_iter, preconditioner=prec, callbacks=callbacks,
+                                           x_true=x_true, **solver_kwargs)
     for method in variants:
-        if method.__name__ == "exact_pcg":                        # the reference's own function, its own call
+        if method.__name__ in batch:
+            trial = batch[method.__name__]
+        elif method.__name__ == "exact_pcg":                        # the reference's own function, its own call
             trial = method(A.astype(np.longdouble), b.astype(np.longdouble), x0.astype(np.longdouble),
                            min(max_iter, N), callbacks=callbacks, x_true=x_true.astype(np.longdouble),
                            preconditioner=prec_long)

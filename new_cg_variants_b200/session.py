@@ -225,6 +225,53 @@ class Session:
         return out.value
 
 
+def solve_batch(items, histories=_lib.HIST_NAMES, return_x=True):
+    """Independent solves side by side on one GPU, in ONE cooperative launch (cgx_batch_run).
+
+    ``items``: sequence of ``(session, variant, b, x0, max_iter[, x_true])``, one distinct Session
+    per entry (same device, same operator kind, same preconditioner mode).  Each entry gets a
+    1/len(items) share of the SMs; its results are bitwise those of ``session.solve(...,
+    path="persistent")`` with the same CTA shape (options ``pers_threads`` / ``pers_ctas``), and
+    ``info["loop_ms"]`` is the duration of the shared launch.
+    Returns ``[(x, {history name: (max_iter,) array}, info), ...]`` as ``Session.solve``."""
+    items = [tuple(it) for it in items]
+    if not items:
+        raise ValueError("solve_batch: no items")
+    sessions, xts = [], []
+    for it in items:
+        if len(it) not in (5, 6):
+            raise ValueError("solve_batch: items are (session, variant, b, x0, max_iter[, x_true])")
+        sess, variant, b, x0, max_iter = it[:5]
+        xt = it[5] if len(it) == 6 else None
+        if variant not in _lib.VARIANT_IDS:
+            raise ValueError(f"solve_batch: unknown variant {variant!r}")
+        sess.load_problem(b, x0, xt)
+        sessions.append(sess)
+        xts.append(xt)
+    mask = 0
+    for h in histories:
+        mask |= _lib.HIST_BITS[h]
+    lib = sessions[0]._lib
+    count = len(items)
+    ctxs = (C.c_void_p * count)(*[s._ctx for s in sessions])
+    variants = np.array([_lib.VARIANT_IDS[it[1]] for it in items], dtype=np.int32)
+    iters = np.array([int(it[4]) for it in items], dtype=np.int32)
+    infos = (_lib.CgxInfo * count)()
+    rc = lib.cgx_batch_run(ctxs, count, _lib.iptr(variants), _lib.iptr(iters), mask, infos)
+    _lib.check(rc, allow_breakdown=True)
+    results = []
+    for sess, it, xt, info in zip(sessions, items, xts, infos):
+        sess.info = info.as_dict()
+        sess._max_iter = int(it[4])
+        x, hist = sess.fetch(want_x=return_x, want_hist=bool(mask))
+        out = {}
+        for i, name in enumerate(_lib.HIST_NAMES):
+            if name in histories and (xt is not None or "error" not in name):
+                out[name] = hist[i].copy()
+        results.append((x, out, sess.info))
+    return results
+
+
 def diagonal_of(A):
     if isinstance(A, PoissonStencil) or sps.issparse(A):
         return np.asarray(A.diagonal(), dtype=np.float64)
