@@ -82,10 +82,10 @@ typedef struct {
   double h2d_bytes;        /* bytes copied host->device by the call */
   double d2h_bytes;        /* bytes copied device->host by the call */
   int64_t kernel_launches; /* kernels of this library launched by the call */
-  int32_t iterations;      /* loop trips executed (max_iter - 1) */
+  int32_t iterations;      /* loop trips executed (max_iter - 1, or stop_iter after a tolerance stop) */
   int32_t breakdown_iter;  /* -1, or first k at which a reduced scalar was non-finite */
   int32_t path;            /* cgx_path actually used */
-  int32_t reserved;
+  int32_t stop_iter;       /* -1, or the iteration k at which the tolerance was met (cgx_set_tolerance) */
 } cgx_info;
 
 typedef struct cgx_ctx cgx_ctx;
@@ -155,6 +155,23 @@ int cgx_get_scalars(cgx_ctx* ctx, double* out9);
  *      "stub_allreduce" = 1 replaces the multi-GPU scalar
  *      exchange by a local stand-in (timing experiment: exposed allreduce time). */
 int cgx_set_option(cgx_ctx* ctx, const char* name, int value);
+/* ---- stop at a relative tolerance (single-GPU contexts: stream path, persistent path, cgx_batch_run).
+ *      rtol = 0 (the default) switches it off: every run then does max_iter - 1 iterations.
+ *      Otherwise 0 < rtol < 1 (anything else, NaN included, is CGX_ERR_ARG), and a run stops at
+ *      stop_iter = the first k >= 1 with nu_k <= rtol^2 * nu_0, where nu_k = r~_k . r_k is the
+ *      recomputed inner product every variant already forms (the M^-1 norm of the updated residual;
+ *      ||r_k||^2 without a preconditioner; never the predicted nu' of PR / M / pipe-*).  Iteration
+ *      stop_iter is completed with all its stages, nothing after it runs.
+ *      Contract: x, the state vectors, cgx_get_scalars and history entries 0 .. stop_iter are bitwise
+ *      those of the same run without a tolerance and with max_iter = stop_iter + 1; later history
+ *      entries are zero.  A run whose tolerance is never met is bitwise the run without one.
+ *      info.stop_iter reports the stop (-1: none) and info.iterations the trips executed; cgx_advance
+ *      (and cgx_advance_stages) after the stop do nothing and return CGX_OK.  A breakdown is reported
+ *      as before; a NaN nu never meets the tolerance.
+ *      Takes effect at the next cgx_begin / cgx_run / cgx_solve_host / cgx_batch_run (per context).
+ *      cgx_begin / cgx_group_begin refuse a rank of a partition with a tolerance set
+ *      (CGX_ERR_UNSUPPORTED); set 0 to run it. */
+int cgx_set_tolerance(cgx_ctx* ctx, double rtol);
 /* timing experiments: 16 %globaltimer stamps written by the last vector pass under
  * cgx_set_option("debug_skip", 2): [0] kernel start, [1] scalars folded, [2] CTA 0 done (ns). */
 int cgx_debug_times(cgx_ctx* ctx, uint64_t* out16);

@@ -29,10 +29,10 @@ class CgxInfo(C.Structure):
     _fields_ = [("loop_ms", C.c_double), ("setup_ms", C.c_double), ("h2d_bytes", C.c_double),
                 ("d2h_bytes", C.c_double), ("kernel_launches", C.c_int64),
                 ("iterations", C.c_int32), ("breakdown_iter", C.c_int32), ("path", C.c_int32),
-                ("reserved", C.c_int32)]
+                ("stop_iter", C.c_int32)]
 
     def as_dict(self):
-        return {f: getattr(self, f) for f, _ in self._fields_ if f != "reserved"}
+        return {f: getattr(self, f) for f, _ in self._fields_}
 
 
 class CgxError(RuntimeError):
@@ -61,6 +61,7 @@ PROTOTYPES = {
     "cgx_get_info": (C.c_int, [_P, C.POINTER(CgxInfo)]),
     "cgx_get_scalars": (C.c_int, [_P, c_double_p]),
     "cgx_set_option": (C.c_int, [_P, C.c_char_p, C.c_int]),
+    "cgx_set_tolerance": (C.c_int, [_P, C.c_double]),
     "cgx_debug_times": (C.c_int, [_P, C.POINTER(C.c_uint64)]),
     "cgx_set_profile": (C.c_int, [_P, C.c_int]),
     "cgx_get_profile": (C.c_int, [_P, C.c_int, c_double_p, C.POINTER(C.c_int64)]),
@@ -131,6 +132,14 @@ def check(rc: int, allow_breakdown: bool = False) -> int:
         return rc
     msg = load().cgx_last_error()
     raise CgxError(rc, msg.decode() if msg else "")
+
+
+def check_tol(tol) -> float:
+    """A relative tolerance as cgx_set_tolerance takes it: 0 (off) or 0 < tol < 1, else ValueError."""
+    t = float(tol)
+    if not (t == 0.0 or 0.0 < t < 1.0):
+        raise ValueError(f"tol must be 0 (off) or satisfy 0 < tol < 1, got {tol!r}")
+    return t
 
 
 def dptr(a: np.ndarray | None):

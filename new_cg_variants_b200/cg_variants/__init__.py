@@ -17,7 +17,10 @@ scaling (identity or Jacobi, figure_gen.py:40-44), otherwise ``NotImplementedErr
 
 Extra keyword arguments understood here (all optional, ignored by the reference):
 ``device=0``, ``path="auto"|"stream"|"persistent"``, ``session=Session`` (reuse an operator
-already resident on the GPU), ``return_info=True`` (adds ``output['_info']``).
+already resident on the GPU), ``return_info=True`` (adds ``output['_info']``), ``tol=`` (stop on the
+GPU at the first k with nu_k <= tol^2 nu_0, nu_k = r~_k . r_k; the histories then have
+``output['stop_iter'] + 1`` entries, and ``output['stop_iter']`` is None when the run went to
+``max_iter``).
 
 ``solve_concurrently(methods, A, b, x0, max_iter, ...)`` runs several of these solvers on the same
 problem in one cooperative launch (figure_gen.py:50-60 runs the nine variants one after another).
@@ -35,7 +38,7 @@ from ..callbacks import CAPTURE_CALLBACKS, DEVICE_HISTORIES
 from ..operators import PoissonStencil, canonical_csr
 from ..session import Session
 
-_OWN_KEYS = ("device", "path", "session", "return_info", "w_replace")
+_OWN_KEYS = ("device", "path", "session", "return_info", "w_replace", "tol")
 
 # ---------------------------------------------------------------------------------------
 # preconditioner probe (SURVEY.md section 8b)
@@ -159,6 +162,7 @@ def _ensure_x_true(A, b, extra, needed):
 
 def _solve(name, tag, A, b, x0, max_iter, preconditioner, callbacks, kwargs):
     own = {k: kwargs.pop(k) for k in _OWN_KEYS if k in kwargs}
+    tol = _lib.check_tol(own["tol"]) if own.get("tol") is not None else 0.0
     device = own.get("device", 0)
     path = own.get("path", "auto")
     n = len(b)
@@ -185,20 +189,23 @@ def _solve(name, tag, A, b, x0, max_iter, preconditioner, callbacks, kwargs):
         sess.set_capture(x="save_x" in names, r=bool(names - {"save_x"}), scalars="lanczos_recurrence" in names)
         try:
             _, hist, info = sess.solve(tag, b, x0, max_iter, x_true=x_true, histories=tuple(dev_hist),
-                                       path=path, return_x=False)
+                                       path=path, return_x=False, tol=tol)
             for h in dev_hist:
                 output[h] = hist[h]
             if capture:
-                _replay_captured(sess, tag, A, b, x0, max_iter, capture, output, kwargs)
+                _replay_captured(sess, tag, A, b, x0, max_iter, capture, output, kwargs, info["stop_iter"])
         finally:
             sess.set_capture()
             sess.set_gv_replace(None)
     else:
         info = _solve_stepwise(sess, tag, A, b, x0, max_iter, x_true, dev_hist, generic, output,
-                               kwargs, path, w_replace if isinstance(plan, str) else None, plan)
+                               kwargs, path, w_replace if isinstance(plan, str) else None, plan, tol)
+    stop = info["stop_iter"]
+    if own.get("tol") is not None:     # (without tol= the output keeps the reference's keys)
+        output["stop_iter"] = stop if stop >= 0 else None
     for cb in ticks:   # leave the terminal as print_k would after the last iteration
         try:
-            cb(output=output, k=max_iter - 1, max_iter=max_iter)
+            cb(output=output, k=stop if stop >= 0 else max_iter - 1, max_iter=max_iter)
         except Exception:
             pass
     if own.get("return_info"):
@@ -206,10 +213,10 @@ def _solve(name, tag, A, b, x0, max_iter, preconditioner, callbacks, kwargs):
     return output
 
 
-def _replay_captured(sess, tag, A, b, x0, max_iter, capture, output, extra):
+def _replay_captured(sess, tag, A, b, x0, max_iter, capture, output, extra, stop=-1):
     """Run the capture-served callbacks once, on the host, from what the GPU recorded during the
-    solve: x_k / r_k rows and the (a, b) the recurrences held after every iteration.  Same keyword
-    protocol as the reference's `callback(**locals())`."""
+    solve: x_k / r_k rows and the (a, b) the recurrences held after every iteration (k = 0 .. stop
+    after a tolerance stop).  Same keyword protocol as the reference's `callback(**locals())`."""
     names = {cb.__name__ for cb in capture}
     X = sess.fetch_capture("x") if "save_x" in names else None
     R = sess.fetch_capture("r") if names - {"save_x"} else None
@@ -217,7 +224,7 @@ def _replay_captured(sess, tag, A, b, x0, max_iter, capture, output, extra):
     predicted = tag in ("pr", "m") or tag.startswith("pipe")
     b_arr = np.asarray(b, dtype=np.float64)
     a_k1 = a_k2 = b_k = b_k1 = 0.0
-    for k in range(max_iter):
+    for k in range(stop + 1 if stop >= 0 else max_iter):
         if k > 0 and sc is not None:
             a_k2, a_k1 = a_k1, sc[0][k - 1]
             b_k1, b_k = b_k, (sc[1][k - 1] if predicted else sc[1][k])
@@ -247,7 +254,7 @@ def _plan_w_replace(w_replace, max_iter):
 
 
 def _solve_stepwise(sess, tag, A, b, x0, max_iter, x_true, dev_hist, generic, output, extra, path,
-                    w_replace=None, plan=None):
+                    w_replace=None, plan=None, tol=0.0):
     """Arbitrary callbacks (and vector-reading GV `w_replace` predicates): step the GPU one
     iteration at a time and hand each callable the reference's keyword set (hs_cg.py:97-98,128-129;
     gv_cg.py:156).  Slow (a device round trip per iteration) but still no CPU arithmetic on the
@@ -259,7 +266,7 @@ def _solve_stepwise(sess, tag, A, b, x0, max_iter, x_true, dev_hist, generic, ou
     if host_pred:
         path = "stream"
     try:
-        sess.begin(tag, max_iter, histories=tuple(dev_hist), path=path)
+        sess.begin(tag, max_iter, histories=tuple(dev_hist), path=path, tol=tol)
     finally:
         sess.set_option("gv_manual", 0)
         sess.set_gv_replace(None)
@@ -309,6 +316,8 @@ def _solve_stepwise(sess, tag, A, b, x0, max_iter, x_true, dev_hist, generic, ou
         for cb in generic:
             cb(**loc)
         x_k1, r_k1 = x_k, r_k
+        if tol and k > 0 and sess.get_info()["stop_iter"] == k:
+            break                                          # the tolerance was met at this iteration
     _, hist = sess.fetch(want_x=False, want_hist=True)
     for h in dev_hist:
         output[h] = hist[_lib.HIST_NAMES.index(h)].copy()
@@ -352,7 +361,8 @@ def solve_concurrently(methods, A, b, x0, max_iter, preconditioner=lambda x: x, 
     Only the four standard callbacks and ``print_k`` are served; any other callback, ``w_replace``,
     ``path=`` or ``session=`` raises ``NotImplementedError`` before the GPU is touched.  One Session
     per method, closed afterwards (the operator cache of the single-method functions is not used).
-    Extra keyword arguments: ``x_true``, ``device=0``, ``return_info=True``."""
+    Extra keyword arguments: ``x_true``, ``device=0``, ``return_info=True``, ``tol=`` (as for the
+    single-method functions; every method stops on its own)."""
     from ..session import solve_batch
     methods = list(methods)
     for key in ("path", "w_replace", "session"):
@@ -373,6 +383,8 @@ def solve_concurrently(methods, A, b, x0, max_iter, preconditioner=lambda x: x, 
                                   f"got {[getattr(cb, '__name__', cb) for cb in generic]}")
     device = kwargs.pop("device", 0)
     return_info = kwargs.pop("return_info", False)
+    tol_arg = kwargs.pop("tol", None)
+    tol = _lib.check_tol(tol_arg) if tol_arg is not None else 0.0
     n = len(b)
     _ensure_x_true(A, b, kwargs, any("error" in h for h in dev_hist))
     x_true = kwargs.get("x_true")
@@ -382,7 +394,7 @@ def solve_concurrently(methods, A, b, x0, max_iter, preconditioner=lambda x: x, 
         for _, _, pre in tags:
             sessions.append(Session(A, dinv=dinv if pre else None, device=device))
         res = solve_batch([(s, tag, b, x0, max_iter, x_true) for s, (_, tag, _) in zip(sessions, tags)],
-                          histories=tuple(dev_hist), return_x=False)
+                          histories=tuple(dev_hist), return_x=False, tol=tol)
     finally:
         for s in sessions:
             s.close()
@@ -391,9 +403,12 @@ def solve_concurrently(methods, A, b, x0, max_iter, preconditioner=lambda x: x, 
         output = {"name": name, "max_iter": max_iter}
         for h in dev_hist:
             output[h] = hist[h]
+        stop = info["stop_iter"]
+        if tol_arg is not None:
+            output["stop_iter"] = stop if stop >= 0 else None
         for cb in ticks:
             try:
-                cb(output=output, k=max_iter - 1, max_iter=max_iter)
+                cb(output=output, k=stop if stop >= 0 else max_iter - 1, max_iter=max_iter)
             except Exception:
                 pass
         if return_info:

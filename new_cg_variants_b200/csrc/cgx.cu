@@ -164,6 +164,8 @@ extern "C" int cgx_ctx_destroy(cgx_ctx* c) {
   cudaFree(c->d_ppart); cudaFree(c->d_pbar); cudaFree(c->d_pout); cudaFree(c->d_prank); cudaFree(c->d_pbatch); cudaFree(c->d_dbg_t); cudaFree(c->d_tma_err);
   for (auto& e : c->ev) cudaEventDestroy(e);
   for (auto& e : c->prof_events) cudaEventDestroy(e);
+  for (auto& e : c->ev_stop) if (e) cudaEventDestroy(e);
+  cudaFreeHost(c->h_stop);
   cudaStreamDestroy(c->own_stream);
   delete c;
   return CGX_OK;
@@ -365,6 +367,7 @@ Args make_args(cgx_ctx* c) {
   g.l2pol = (c->l2_keep == 1 || (c->l2_keep < 0 && c->n > 0 && (size_t)c->n * 8 * 6 < ((size_t)96 << 20))) ? kL2EvictLast : 0;
   g.dbg = c->dbg;
   g.dbg_t = c->d_dbg_t;
+  g.tol_on = c->run_tol > 0.0 ? 1 : 0;
   return g;
 }
 
@@ -572,13 +575,16 @@ void launch_hist_consume(cgx_ctx* c, Args g) {
   hist_consume_kernel<<<1, 32, 0, c->stream>>>(g);
   c->launches++;
 }
-static void launch_dot(cgx_ctx* c, const double* u, const double* v, const double* dinv, int slot) {
+// stop != nullptr: a step of iteration k, skipped on the device after a tolerance stop
+static void launch_dot(cgx_ctx* c, const double* u, const double* v, const double* dinv, int slot,
+                       const Scal* stop = nullptr, int k = 0) {
   dot_kernel<<<grid_for(c, c->n), kBlock, 0, c->stream>>>(u, v, dinv, c->n, c->d_sc + c->scpar, slot,
-                                                          c->d_partials, c->d_ticket);
+                                                          c->d_partials, c->d_ticket, stop, k);
   c->launches++;
 }
-static void launch_scale(cgx_ctx* c, const double* dinv, const double* v, double* out) {
-  scale_kernel<<<grid_for(c, c->n), kBlock, 0, c->stream>>>(dinv, v, out, c->n);
+static void launch_scale(cgx_ctx* c, const double* dinv, const double* v, double* out,
+                         const Scal* stop = nullptr, int k = 0) {
+  scale_kernel<<<grid_for(c, c->n), kBlock, 0, c->stream>>>(dinv, v, out, c->n, stop, k);
   c->launches++;
 }
 
@@ -615,17 +621,18 @@ void launch_capture(cgx_ctx* c, const Args& g) {
   if (c->capture & CGX_CAPTURE_X) cudaMemcpyAsync(c->d_cap[0] + (size_t)g.k * c->n, c->vec[V_X], bytes, cudaMemcpyDeviceToDevice, c->stream);
   if (c->capture & CGX_CAPTURE_R) cudaMemcpyAsync(c->d_cap[1] + (size_t)g.k * c->n, c->vec[V_R], bytes, cudaMemcpyDeviceToDevice, c->stream);
   if (c->capture & CGX_CAPTURE_SCALARS) {
-    capture_scalars_kernel<<<1, 32, 0, c->stream>>>(c->d_sc, c->d_cap[2], g.k, c->hist_len);
+    capture_scalars_kernel<<<1, 32, 0, c->stream>>>(c->d_sc, c->d_cap[2], g.k, c->hist_len, g.tol_on);
     c->launches++;
   }
 }
 
 // GV residual replacement at iteration g.k, between the vector pass and t = A wt
 static void launch_gv_replace(cgx_ctx* c, Args g) {
+  const Scal* stop = g.tol_on ? c->d_sc : nullptr;
   launch_spmv<SP_PLAIN, 0, false>(c, g, c->vec[V_R], c->vec[V_W]);          // w = A r        gv_cg.py:158
-  launch_scale(c, c->d_dinv, c->vec[V_W], c->vec[V_WT]);                    // wt = M w       :160
-  launch_dot(c, c->vec[V_W], c->vec[V_RT], nullptr, 5);                     // eta = w . rt   :163
-  gv_refinalize_kernel<<<1, 32, 0, c->stream>>>(c->d_sc, g.k);              // mu, a          :169-170
+  launch_scale(c, c->d_dinv, c->vec[V_W], c->vec[V_WT], stop, g.k);         // wt = M w       :160
+  launch_dot(c, c->vec[V_W], c->vec[V_RT], nullptr, 5, stop, g.k);          // eta = w . rt   :163
+  gv_refinalize_kernel<<<1, 32, 0, c->stream>>>(c->d_sc, g.k, g.tol_on);    // mu, a          :169-170
   c->launches++;
 }
 
@@ -724,6 +731,7 @@ static void build_init_steps(cgx_ctx* c, int variant, const VariantInfo& vi, Ste
     });
   }
   const int cls = vi.cls, meur = vi.meurant ? 1 : 0;
+  const double tol = c->run_tol;
   st.push_back([=]() {
     Args g = make_args(c);
     g.scpar = c->scpar;
@@ -731,7 +739,7 @@ static void build_init_steps(cgx_ctx* c, int variant, const VariantInfo& vi, Ste
       g.pend_e[0] = c->epoch;
       if (c->dist.mode == 2) cudaStreamWaitEvent(c->stream, c->ev_red[c->epoch % kSlots], 0);
     }
-    init_scalars_kernel<<<1, 32, 0, c->stream>>>(g, cls, meur);
+    init_scalars_kernel<<<1, 32, 0, c->stream>>>(g, cls, meur, tol);
     c->launches++;
   });
 }
@@ -855,7 +863,16 @@ static int begin_prepare(cgx_ctx* c, int variant, int max_iter, unsigned hist_ma
     return fail(CGX_ERR_ARG, "cgx_begin: unknown path %d", path);
   if (c->dist.world > 1 && !c->dist_ready)
     return fail(CGX_ERR_ARG, "cgx_begin: cgx_dist_commit has not been called on this rank");
+  if (c->dist.world > 1 && c->tol > 0.0)
+    return fail(CGX_ERR_UNSUPPORTED, "cgx_begin: a tolerance stops single-GPU solves only (rank %d of a partition has one set)",
+                c->dist.rank);
   CU(cudaSetDevice(c->device));
+  if (c->tol > 0.0 && !c->h_stop) {
+    CU(cudaHostAlloc(&c->h_stop, 2 * sizeof(int), cudaHostAllocDefault));
+    for (int i = 0; i < 2; ++i) CU(cudaEventCreateWithFlags(&c->ev_stop[i], cudaEventDisableTiming));
+  }
+  c->run_tol = c->tol;
+  c->stop_k = -1;
   const bool prec = c->d_dinv != nullptr;
   const VariantInfo vi = variant_info(variant, prec);
   hist_mask &= CGX_HIST_ALL;
@@ -954,6 +971,10 @@ static int check_device_flags(cgx_ctx* c, const char* who) {
 
 // Lockstep driver: `count` contexts (ranks of one partitioned problem, or a single context).
 static int group_begin(cgx_ctx** cs, int count, int variant, int max_iter, unsigned hist_mask, int path) {
+  for (int i = 0; i < count; ++i)       // (before any rank has enqueued anything)
+    if (cs[i] && cs[i]->dist.world > 1 && cs[i]->tol > 0.0)
+      return fail(CGX_ERR_UNSUPPORTED, "cgx_begin: a tolerance stops single-GPU solves only (rank %d of a partition has one set)",
+                  cs[i]->dist.rank);
   bool same_device = count > 1;
   for (int i = 1; i < count; ++i) same_device = same_device && cs[i]->device == cs[0]->device;
   for (int i = 0; i < count; ++i) {
@@ -1004,11 +1025,24 @@ static int group_begin(cgx_ctx** cs, int count, int variant, int max_iter, unsig
   return CGX_OK;
 }
 
+// After the stream has drained: adopt the stop_k the device decided (runs with a tolerance only).
+static int read_stop(cgx_ctx* c) {
+  if (c->run_tol <= 0.0) return CGX_OK;
+  int s = -1;
+  CU(cudaMemcpy(&s, &c->d_sc[c->scpar].stop_k, sizeof(int), cudaMemcpyDeviceToHost));
+  c->stop_k = s;
+  // the fused PR kernel swaps the buffers of p, s, rt once per iteration it runs; the launches after the
+  // stop returned at entry, so the current buffers are those of iteration stop_k (cgx_cur_vec)
+  if (s >= 0 && c->pr_fused) c->fpar = s & 1;
+  return CGX_OK;
+}
+
 static int group_advance(cgx_ctx** cs, int count, int niter) {
   for (int i = 0; i < count; ++i)
     if (!cs[i] || !cs[i]->ran) return fail(CGX_ERR_ARG, "cgx_advance: call cgx_begin first");
   if (niter < 0) return fail(CGX_ERR_ARG, "cgx_advance: niter must be >= 0");
   cgx_ctx* c0 = cs[0];
+  if (c0->stop_k >= 0) return CGX_OK;   // the tolerance was met: nothing left to run
   const int last = std::min(c0->max_iter - 1, c0->cur_k + niter);
   std::vector<i64> l0(count);
   std::vector<Args> gs(count);
@@ -1032,7 +1066,17 @@ static int group_advance(cgx_ctx** cs, int count, int niter) {
   } else {
     const int ns = iter_stage_count(c0);
     if (c0->cur_stage != 0) return fail(CGX_ERR_ARG, "cgx_advance: an iteration is half done (cgx_advance_stages); finish it first");
-    for (int k = c0->cur_k + 1; k <= last; ++k)
+    // with a tolerance (single contexts only): chunks of kTolChunk iterations, each followed by a copy of
+    // stop_k into pinned slot j & 1; chunk j is enqueued once chunk j - 2 has completed and did not stop
+    const bool poll = c0->run_tol > 0.0;
+    const int first = c0->cur_k + 1;
+    for (int k = first; k <= last; ++k) {
+      const int j = (k - first) / kTolChunk;
+      const bool chunk_start = (k - first) % kTolChunk == 0, chunk_end = (k - first) % kTolChunk == kTolChunk - 1 || k == last;
+      if (poll && chunk_start && j >= 2) {
+        CU(cudaEventSynchronize(c0->ev_stop[j & 1]));
+        if (c0->h_stop[j & 1] >= 0) break;
+      }
       for (int s = 0; s < ns; ++s)
         for (int i = 0; i < count; ++i) {
           if (count > 1) cudaSetDevice(cs[i]->device);
@@ -1041,6 +1085,11 @@ static int group_advance(cgx_ctx** cs, int count, int niter) {
             launch_gv_replace(cs[i], gs[i]);
           iter_stage(cs[i], s, gs[i]);
         }
+      if (poll && chunk_end) {
+        CU(cudaMemcpyAsync(&c0->h_stop[j & 1], &c0->d_sc[c0->scpar].stop_k, sizeof(int), cudaMemcpyDeviceToHost, c0->stream));
+        CU(cudaEventRecord(c0->ev_stop[j & 1], c0->stream));
+      }
+    }
     for (int i = 0; i < count; ++i) {
       if (count > 1) cudaSetDevice(cs[i]->device);
       const VariantInfo vi = variant_info(cs[i]->variant, cs[i]->d_dinv != nullptr);
@@ -1065,7 +1114,9 @@ static int group_advance(cgx_ctx** cs, int count, int niter) {
     if (rc) return rc;
     if (ran_pers) { rc = pers_collect(c); if (rc) return rc; }
     c->launches_run += c->launches - l0[i];
-    c->cur_k = std::max(c->cur_k, last);
+    rc = read_stop(c);
+    if (rc) return rc;
+    c->cur_k = c->stop_k >= 0 ? c->stop_k : std::max(c->cur_k, last);
   }
   return CGX_OK;
 }
@@ -1258,7 +1309,9 @@ static int batch_run(cgx_ctx** cs, int count, const int* variants, const int* ma
     if (rc) return rc;
     if (max_iters[i] > 1) { rc = pers_collect(c); if (rc) return rc; }
     c->launches_run += c->launches - l0[i];
-    c->cur_k = c->max_iter - 1;
+    rc = read_stop(c);
+    if (rc) return rc;
+    c->cur_k = c->stop_k >= 0 ? c->stop_k : c->max_iter - 1;
     rc = cgx_get_info(c, &infos[i]);
     if (rc) return rc;
     broke = broke || infos[i].breakdown_iter >= 0;
@@ -1293,7 +1346,7 @@ extern "C" int cgx_get_info(cgx_ctx* c, cgx_info* info) {
   info->iterations = c->cur_k;
   info->breakdown_iter = h.breakdown;
   info->path = c->path;
-  info->reserved = 0;
+  info->stop_iter = c->stop_k;
   return CGX_OK;
 }
 
@@ -1329,6 +1382,14 @@ extern "C" int cgx_set_option(cgx_ctx* c, const char* name, int value) {
     return CGX_OK;
   }
   return fail(CGX_ERR_ARG, "cgx_set_option: unknown option '%s'", name);
+}
+
+extern "C" int cgx_set_tolerance(cgx_ctx* c, double rtol) {
+  if (!c) return fail(CGX_ERR_ARG, "cgx_set_tolerance: ctx is NULL");
+  if (!(rtol == 0.0 || (rtol > 0.0 && rtol < 1.0)))
+    return fail(CGX_ERR_ARG, "cgx_set_tolerance: rtol must be 0 (off) or in (0, 1), got %g", rtol);
+  c->tol = rtol;
+  return CGX_OK;
 }
 
 // timing experiments: the 16 %globaltimer stamps kernels wrote under option debug_skip & 2
@@ -1394,6 +1455,7 @@ extern "C" int cgx_advance_stages(cgx_ctx* c, int nstages) {
   if (!c || !c->ran || nstages < 0) return fail(CGX_ERR_ARG, "cgx_advance_stages: call cgx_begin first");
   if (c->path != CGX_PATH_STREAM || c->dist.world > 1)
     return fail(CGX_ERR_UNSUPPORTED, "cgx_advance_stages: single-GPU stream path only");
+  if (c->stop_k >= 0) return CGX_OK;
   CU(cudaSetDevice(c->device));
   const int ns = iter_stage_count(c);
   Args g = make_args(c);
@@ -1406,6 +1468,10 @@ extern "C" int cgx_advance_stages(cgx_ctx* c, int nstages) {
   CU(cudaStreamSynchronize(c->stream));
   CU(cudaGetLastError());
   c->launches_run += c->launches - l0;
+  int rc = read_stop(c);
+  if (rc) return rc;
+  if (c->stop_k >= 0 && c->stop_k > c->cur_k) c->stop_k = -1;      // iteration stop_k is not complete yet
+  if (c->stop_k >= 0) { c->cur_k = c->stop_k; c->cur_stage = 0; }
   return check_device_flags(c, "cgx_advance_stages");
 }
 extern "C" int cgx_gv_replace_now(cgx_ctx* c) {

@@ -29,7 +29,8 @@ struct Scal {
   double nu, nu1, mu, eta, del, gam;
   double tmp[8];      // initialisation dot products
   int breakdown;      // -1, or first k with a non-finite alpha/beta
-  int pad;
+  int stop_k;         // -1, or first k >= 1 with nu_k <= thr (cgx_set_tolerance); the run ends after iteration stop_k
+  double thr;         // tol^2 * nu_0, or NaN when no tolerance is set (no nu satisfies the test)
 };
 
 // ---- arithmetic that must mirror numpy's two-rounding elementwise expressions ---------
@@ -199,6 +200,16 @@ __device__ __forceinline__ void grid_last_finalize(unsigned* __restrict__ ticket
 
 __device__ __forceinline__ void note_breakdown(Scal* sc, int k, double a, double b) {
   if (sc->breakdown < 0 && !(isfinite(a) && isfinite(b))) sc->breakdown = k;
+}
+// Called wherever nu_k is assigned: the natural norm of the updated residual, r~_k . r_k, against
+// tol^2 nu_0.  A NaN nu (or threshold) never satisfies the test.
+__device__ __forceinline__ void note_stop(Scal* sc, int k) {
+  if (sc->stop_k < 0 && k >= 1 && sc->nu <= sc->thr) sc->stop_k = k;
+}
+// A launch that belongs to iteration k after the one at which the tolerance was met does nothing.
+__device__ __forceinline__ bool past_stop(const Scal* sc, int k) {
+  const int s = sc->stop_k;
+  return s >= 0 && k > s;
 }
 
 // =====================================================================================

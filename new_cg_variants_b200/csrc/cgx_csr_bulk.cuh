@@ -115,6 +115,7 @@ csr_bulk_kernel(const CsrOp A, const int* __restrict__ row_blocks, const int* __
   __shared__ CbMeta meta[kCbMaxRing];
   __shared__ double sh_ylong[2];                     // running sum of a long row, handed from chunk to chunk
   __shared__ int sh_long_done;                       // chunks of long rows summed so far
+  if (after_stop(g)) return;
   const int tid = threadIdx.x;
   const int R = ring;
   const int nsum = ((int)blockDim.x - kCbSum0) / 32;

@@ -172,6 +172,11 @@ struct cgx_ctx {
   std::map<std::pair<const void*, size_t>, int> occ;   // ctx_occupancy cache (per device)
   int* d_tma_err = nullptr;                // set by a TMA wait that expired (mbar_wait)
   int variant = 0, max_iter = 0, cur_k = 0, path = CGX_PATH_STREAM;
+  // relative tolerance (cgx_set_tolerance): requested, and in force for the current run
+  double tol = 0.0, run_tol = 0.0;
+  int stop_k = -1;                         // host copy of Scal::stop_k once the run has stopped
+  int* h_stop = nullptr;                   // pinned: stop_k after chunk j of the stream loop, slot j & 1
+  cudaEvent_t ev_stop[2] = {nullptr, nullptr};
   i64 launches_run = 0;
   double setup_ms = 0.0, loop_ms = 0.0;
 };
@@ -243,6 +248,11 @@ inline cudaError_t launch_k(void (*kern)(KArgs...), int grid, int block, size_t 
 inline bool use_pdl(const cgx_ctx* c) { return c->pdl_mode == 2 || (c->pdl_mode == 1 && c->dist.world <= 1); }
 
 inline size_t tma_smem_bytes(int nv) { return stencil_smem_bytes(nv); }
+
+// Stream path with a tolerance: iterations issued between two looks at stop_k.  The host waits for chunk
+// j - 2 before it enqueues chunk j, so the queue stays at least a chunk deep and the launches issued after
+// the stop (all of which return at entry) are at most two chunks' worth.
+constexpr int kTolChunk = 32;
 
 // kernel launches ("stages") of one iteration without the instrumentation
 // (a CSR row partition adds one stage: the gather-and-push of the SpMV input's ghost entries)

@@ -101,9 +101,15 @@ struct Args {
   int* errflag;                    // device word set by a bounded in-kernel wait that expired
   unsigned long long l2pol;        // 0, or an L2 cache-policy word for the state-vector accesses (kL2EvictLast)
   double* gscr;                    // fused PR kernel on a partition: [plane] new p of the ghost plane above the slab
+  int tol_on;                      // a tolerance is set: launches of iterations after sc->stop_k return at entry
   int dbg;                         // timing experiments (cgx_set_option "debug_skip"): 1 = no halo traffic, 2 = time stamps
   u64* dbg_t;                      // dbg & 2: CTA 0 writes %globaltimer at kernel start / after the scalar fold / at its end
 };
+
+// Every kernel of the iteration loop starts with this test (after griddepcontrol.wait where the kernel
+// is launched with programmatic serialisation: stop_k is written by an earlier kernel).  g.sc->stop_k was
+// written before the launch, so every CTA takes the same branch.
+__device__ __forceinline__ bool after_stop(const Args& g) { return g.tol_on && past_stop(g.sc, g.k); }
 
 // An SpMV input vector: the owned slab and (multi-GPU) the ghost planes below and above.
 struct VecIn { const double* v; const double* lo; const double* hi; };
@@ -153,13 +159,16 @@ __device__ __forceinline__ double predict_beta(bool meurant, double nu, double a
 }
 
 // Scalar recurrences that close a fused reduction (run by one thread with the grid -- or,
-// multi-GPU, the all-rank -- totals).  kind: FK_* of cgx_common.cuh.
-__device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc, const double* acc, int k) {
+// multi-GPU, the all-rank -- totals).  kind: FK_* of cgx_common.cuh.  stop_test: look for the
+// tolerance stop (partitions, which refuse a tolerance, leave it out of their scalar fold).
+__device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc, const double* acc, int k,
+                                               bool stop_test = true) {
   if (kind == FK_HS_NU) {                    // hs_cg.py:120-121
     const double nu1 = sc->nu;
     sc->nu1 = nu1; sc->nu = acc[0];
     sc->b = div_(acc[0], nu1);
     note_breakdown(sc, k, sc->a, sc->b);
+    if (stop_test) note_stop(sc, k);
   } else if (kind == FK_HS_MU) {             // hs_cg.py:124-125
     sc->mu = acc[0];
     sc->a1 = sc->a; sc->a = div_(sc->nu, acc[0]);
@@ -171,8 +180,10 @@ __device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc,
     sc->nu1 = nu1; sc->nu = nu; sc->eta = eta; sc->b = bb; sc->mu = mu;
     sc->a1 = a1; sc->a = div_(nu, mu);
     note_breakdown(sc, k, sc->a, bb);
+    if (stop_test) note_stop(sc, k);
   } else if (kind == FK_PR_NU) {             // pr_cg.py:157 (consumed by the SpMV pass)
     sc->nu1 = sc->nu; sc->nu = acc[0];
+    if (stop_test) note_stop(sc, k);
   } else if (kind == FK_PR_SP) {             // pr_cg.py:154-158 then :149-150
     const double mu = acc[0], del = acc[1], gam = acc[2], nu = sc->nu;
     sc->mu = mu; sc->del = del; sc->gam = gam;
@@ -187,6 +198,7 @@ __device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc,
     sc->a1 = sc->a; sc->a = an;
     sc->b = predict_beta(meurant, nu, an, del, gam);
     note_breakdown(sc, k, an, sc->b);
+    if (stop_test) note_stop(sc, k);
   }
 }
 
@@ -290,13 +302,17 @@ __device__ __forceinline__ void dist_fold(const Args& g, bool meurant, double* s
           dist_totals(g, g.pend_e[q], fk_width(g.pend_kind[q]), acc);
         }
         if (stamp) g.dbg_t[5 + 2 * q] = (u64)clock64();
-        apply_finalize(g.pend_kind[q], meurant, &s, acc, g.pend_k[q]);
+        apply_finalize(g.pend_kind[q], meurant, &s, acc, g.pend_k[q], false);
         if (stamp) g.dbg_t[6 + 2 * q] = (u64)clock64();
       }
     }
     if (threadIdx.x == 0) {
       sh_ab[0] = s.a; sh_ab[1] = s.b;
-      if (blockIdx.x == 0 && g.npend) g.sc[g.scpar ^ 1] = s;
+      if (blockIdx.x == 0 && g.npend) {          // (tmp[] is initialisation scratch: not carried over)
+        Scal* o = &g.sc[g.scpar ^ 1];
+        o->a = s.a; o->a1 = s.a1; o->b = s.b; o->nu = s.nu; o->nu1 = s.nu1; o->mu = s.mu; o->eta = s.eta;
+        o->del = s.del; o->gam = s.gam; o->breakdown = s.breakdown; o->stop_k = s.stop_k; o->thr = s.thr;
+      }
     }
   }
   if (stamp) g.dbg_t[9] = (u64)clock64();
@@ -542,6 +558,7 @@ __global__ void __launch_bounds__(kBlock) ew_kernel(const Args g) {
   const bool stamp = (g.dbg & 2) && blockIdx.x == 0 && threadIdx.x == 0;
   pdl_launch_dependents();
   pdl_wait();                          // nothing of the previous kernel's data is touched before this
+  if (after_stop(g)) return;
   if (stamp) g.dbg_t[0] = (u64)clock64();
   if (dist) {
     const i64 rot0 = (g.hout_n > 0 && g.d.has_hi) ? nv - (g.d.plane >> 1) : 0;
@@ -661,6 +678,7 @@ __global__ void __launch_bounds__(kBlock) spmv_kernel(const Op A, const Args g, 
                                                      const VecIn in1, double* vout) {
   constexpr bool SL = Op::kSlab;
   constexpr int NV = SpTraits<MODE>::NV;
+  if (after_stop(g)) return;
   halo_wait_all(g, NV);
   double red[kNRed] = {0.0, 0.0, 0.0, 0.0};
   const i64 n = g.n, pl = g.d.plane;
@@ -719,6 +737,7 @@ csr_stream_kernel(const CsrOp A, const int* __restrict__ row_blocks, const int* 
   int* sm_rp = reinterpret_cast<int*>(sm_d + (size_t)S * csr_slot_doubles(NV));         // [S][kBlock + 4] row extents
   CsrSlotMeta* sm_meta = reinterpret_cast<CsrSlotMeta*>(sm_rp + S * (kBlock + 4));      // [S]
   __shared__ __align__(8) uint64_t full_bar[3], empty_bar[3];
+  if (after_stop(g)) return;
   const int tid = threadIdx.x;
   if (tid == 0) {
     for (int s = 0; s < S; ++s) { mbar_init(&full_bar[s], kCsrLoaders / 32); mbar_init(&empty_bar[s], 1); }
@@ -936,6 +955,7 @@ template <class Op, bool HAS_XTRUE>
 __global__ void __launch_bounds__(kBlock) instrument_kernel(const Op A, const Args g, const VecIn xin,
                                                            const VecIn xtin) {
   constexpr bool SL = Op::kSlab;
+  if (after_stop(g)) return;
   if (HAS_XTRUE && g.d.world > 1 && threadIdx.x == 0 && g.d.csr) {
     csr_wait_channel(g, 3, g.xt_par, g.xt_epoch);
   } else if (HAS_XTRUE && g.d.world > 1 && threadIdx.x == 0) {
@@ -1024,9 +1044,12 @@ static __global__ void __launch_bounds__(kBlock) csr_halo_push_kernel(const Args
 // -------------------------------------------------------------------------------------
 // Small helpers used only by the (non-timed) initialisation.
 // -------------------------------------------------------------------------------------
+// stop != nullptr: a step of GV residual replacement at iteration k (nothing to do after the stop)
 static __global__ void __launch_bounds__(kBlock) scale_kernel(const double* __restrict__ dinv,
                                                       const double* __restrict__ v,
-                                                      double* __restrict__ out, i64 n) {
+                                                      double* __restrict__ out, i64 n,
+                                                      const Scal* stop, int k) {
+  if (stop && past_stop(stop, k)) return;
   const i64 stride = (i64)gridDim.x * kBlock;
   for (i64 i = (i64)blockIdx.x * kBlock + threadIdx.x; i < n; i += stride)
     out[i] = dinv ? mul_(dinv[i], v[i]) : v[i];
@@ -1037,7 +1060,8 @@ static __global__ void __launch_bounds__(kBlock) dot_kernel(const double* __rest
                                                     const double* __restrict__ v,
                                                     const double* __restrict__ dinv, i64 n,
                                                     Scal* sc, int slot, double* partials,
-                                                    unsigned* ticket) {
+                                                    unsigned* ticket, const Scal* stop, int k) {
+  if (stop && past_stop(stop, k)) return;
   double red[1] = {0.0};
   const i64 stride = (i64)gridDim.x * kBlock;
   for (i64 i = (i64)blockIdx.x * kBlock + threadIdx.x; i < n; i += stride) {
@@ -1048,13 +1072,14 @@ static __global__ void __launch_bounds__(kBlock) dot_kernel(const double* __rest
 }
 
 // capture of the scalars after iteration k: out[0][k] = a, out[1][k] = b
-static __global__ void capture_scalars_kernel(const Scal* sc, double* out, int k, int len) {
+static __global__ void capture_scalars_kernel(const Scal* sc, double* out, int k, int len, int tol_on) {
+  if (tol_on && past_stop(sc, k)) return;
   if (threadIdx.x == 0) { out[k] = sc->a; out[len + k] = sc->b; }
 }
 // GV residual replacement (gv_cg.py:156-158, then :162-170 with the new w): eta was re-formed from the
 // replaced w (tmp[5]); nu, nu1, b are those of the vector pass
-static __global__ void gv_refinalize_kernel(Scal* sc, int k) {
-  if (threadIdx.x != 0) return;
+static __global__ void gv_refinalize_kernel(Scal* sc, int k, int tol_on) {
+  if (threadIdx.x != 0 || (tol_on && past_stop(sc, k))) return;
   const double eta = sc->tmp[5];
   sc->eta = eta;
   sc->mu = sub_(eta, mul_(div_(sc->b, sc->a1), sc->nu));
@@ -1082,7 +1107,8 @@ static __global__ void push_tmp_kernel(const Args g) {
 // Initial scalars from the initialisation dots.  tmp: 0 nu, 1 mu, 2 eta, 3 delta, 4 gamma.
 // variant_class: 0 HS, 1 CG/GV (mu := p.s), 2 PR/M/pipe (predict first beta).
 // Multi-GPU (g.d.world > 1): tmp[] first becomes the all-rank total of epoch pend_e[0].
-static __global__ void init_scalars_kernel(const Args g, int variant_class, int meurant) {
+// tol > 0: the relative tolerance of cgx_set_tolerance (threshold tol^2 nu_0); 0: none.
+static __global__ void init_scalars_kernel(const Args g, int variant_class, int meurant, double tol) {
   if (threadIdx.x != 0) return;
   Scal* sc = g.sc + g.scpar;
   if (g.d.world > 1) {
@@ -1109,6 +1135,8 @@ static __global__ void init_scalars_kernel(const Args g, int variant_class, int 
   sc->a = div_(nu, mu);
   sc->b = 0.0;
   sc->breakdown = -1;
+  sc->stop_k = -1;
+  sc->thr = tol > 0.0 ? mul_(mul_(tol, tol), nu) : nan("");
   if (variant_class == 2) sc->b = predict_beta(meurant != 0, nu, sc->a, sc->del, sc->gam);
   note_breakdown(sc, 0, sc->a, sc->b);
 }

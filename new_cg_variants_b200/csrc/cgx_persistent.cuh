@@ -281,6 +281,7 @@ __device__ __forceinline__ void persistent_body(const PersRank<Op>& pr, const Pe
     const Scal* i0 = &g.sc[dist ? g.scpar : 0];
     s.a = i0->a; s.a1 = i0->a1; s.b = i0->b; s.nu = i0->nu; s.nu1 = i0->nu1; s.mu = i0->mu; s.eta = i0->eta;
     s.del = i0->del; s.gam = i0->gam; s.breakdown = i0->breakdown;
+    s.stop_k = i0->stop_k; s.thr = i0->thr;
   }
   u64 nbar = 0, epoch = pr.epoch0;
   u64 hep[kChan];
@@ -580,6 +581,9 @@ __device__ __forceinline__ void persistent_body(const PersRank<Op>& pr, const Pe
     }
     if (hist) sync_point(red, NR8{}, SpTraits<SP>::FK, k, true, 0, 0);
     else if constexpr (NRS > 0) sync_point(red, std::integral_constant<int, NRS>{}, SpTraits<SP>::FK, k, false, 0, 0);
+    // a tolerance was met in this iteration: every CTA formed the same stop_k from the same totals at a
+    // sync point of this iteration and leaves here, after the last one, so none waits on a counter
+    if (s.stop_k >= 0) break;
   }
   fold_pending();
 
@@ -601,7 +605,7 @@ __device__ __forceinline__ void persistent_body(const PersRank<Op>& pr, const Pe
   if (cta == 0 && tid == 0) {
     Scal* o = &g.sc[dist ? g.scpar : 0];           // (tmp[] is initialisation scratch: not kept live)
     o->a = s.a; o->a1 = s.a1; o->b = s.b; o->nu = s.nu; o->nu1 = s.nu1; o->mu = s.mu; o->eta = s.eta;
-    o->del = s.del; o->gam = s.gam; o->breakdown = s.breakdown;
+    o->del = s.del; o->gam = s.gam; o->breakdown = s.breakdown; o->stop_k = s.stop_k;
     pr.out->epoch = epoch;
     for (int c = 0; c < kChan; ++c) pr.out->hepoch[c] = hep[c];
   }

@@ -66,6 +66,11 @@ pr_fused_kernel(const __grid_constant__ CUtensorMap tm_p, const __grid_constant_
   __shared__ __align__(8) uint64_t full_bar[kFStages], empty_bar[kFStages];
 
   const int tid = threadIdx.x;
+  if (g.tol_on) {                      // stop_k is visible only after the wait: no prologue overlap then
+    pdl_launch_dependents();
+    pdl_wait();
+    if (after_stop(g)) return;
+  }
   if (tid == 0) {
 #pragma unroll
     for (int s = 0; s < kFStages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], kFConsumers / 32); }

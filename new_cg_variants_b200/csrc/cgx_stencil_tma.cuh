@@ -85,6 +85,11 @@ stencil_tma_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constan
   __shared__ __align__(8) uint64_t full_bar[R], empty_bar[R];
 
   const int tid = threadIdx.x;
+  if (g.tol_on) {                      // stop_k is visible only after the wait: no prologue overlap then
+    pdl_launch_dependents();
+    pdl_wait();
+    if (after_stop(g)) return;
+  }
   if (tid == 0) {
 #pragma unroll
     for (int s = 0; s < R; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], kSConsumers / 32); }

@@ -34,6 +34,7 @@ class Session:
         _lib.check(self._lib.cgx_ctx_create(int(device), C.byref(self._ctx)))
         self.device = int(device)
         self.info = None
+        self._tol = 0.0
         if isinstance(A, PoissonStencil):
             self.kind = "stencil"
             self.n = A.shape[0]
@@ -77,6 +78,28 @@ class Session:
             _lib.check(self._lib.cgx_set_jacobi_host(self._ctx, _lib.dptr(d), self.n))
             self.prec = True
 
+    def set_tolerance(self, tol):
+        """Stop every later run once nu_k <= tol^2 nu_0 (nu_k = r~_k . r_k); 0 switches it off.
+        Takes effect at the next begin / run / solve (include/cgx.h cgx_set_tolerance)."""
+        t = _lib.check_tol(tol)
+        _lib.check(self._lib.cgx_set_tolerance(self._ctx, t))
+        self._tol = t
+
+    def _with_tol(self, tol, call):
+        """Run `call()` with tolerance `tol` (None: the session's own), then restore the session's."""
+        if tol is None:
+            return call()
+        prev = self._tol
+        self.set_tolerance(tol)
+        try:
+            return call()
+        finally:
+            self.set_tolerance(prev)
+
+    def _stop(self):
+        """stop_iter of the last run (-1: it ran to max_iter)."""
+        return self.get_info()["stop_iter"]
+
     def load_problem(self, b, x0, x_true=None):
         b = _f64(b, self.n, "b")
         x0 = _f64(x0, self.n, "x0")
@@ -89,25 +112,33 @@ class Session:
         _lib.check(self._lib.cgx_load_problem_dev(self._ctx, b_ptr, x0_ptr, x_true_ptr, self.n))
 
     # -- running ---------------------------------------------------------------------
-    def run(self, variant, max_iter, histories=(), path="auto"):
-        """Iterate on the loaded problem; returns the info dict (device timings etc.)."""
+    def run(self, variant, max_iter, histories=(), path="auto", tol=None):
+        """Iterate on the loaded problem; returns the info dict (device timings etc.).
+        ``tol``: relative tolerance for this run (see ``set_tolerance``); ``info["stop_iter"]``
+        is the iteration it stopped at, or -1."""
+        if tol is not None:
+            _lib.check_tol(tol)
         mask = 0
         for h in histories:
             mask |= _lib.HIST_BITS[h]
         info = _lib.CgxInfo()
-        rc = self._lib.cgx_run(self._ctx, _lib.VARIANT_IDS[variant], int(max_iter), mask,
-                               _lib.PATHS[path], C.byref(info))
+        rc = self._with_tol(tol, lambda: self._lib.cgx_run(self._ctx, _lib.VARIANT_IDS[variant], int(max_iter), mask,
+                                                           _lib.PATHS[path], C.byref(info)))
         _lib.check(rc, allow_breakdown=True)
         self.info = info.as_dict()
         self._max_iter = int(max_iter)
         return self.info
 
-    def begin(self, variant, max_iter, histories=(), path="auto"):
+    def begin(self, variant, max_iter, histories=(), path="auto", tol=None):
+        """Initialise a stepwise solve (``advance``); ``tol`` as in ``run``.  ``advance`` after the
+        tolerance stop does nothing."""
+        if tol is not None:
+            _lib.check_tol(tol)
         mask = 0
         for h in histories:
             mask |= _lib.HIST_BITS[h]
-        _lib.check(self._lib.cgx_begin(self._ctx, _lib.VARIANT_IDS[variant], int(max_iter), mask,
-                                       _lib.PATHS[path]))
+        _lib.check(self._with_tol(tol, lambda: self._lib.cgx_begin(self._ctx, _lib.VARIANT_IDS[variant], int(max_iter),
+                                                                   mask, _lib.PATHS[path])))
         self._max_iter = int(max_iter)
 
     def advance(self, niter=1):
@@ -143,10 +174,14 @@ class Session:
         _lib.check(self._lib.cgx_set_capture(self._ctx, (1 if x else 0) | (2 if r else 0) | (4 if scalars else 0)))
 
     def fetch_capture(self, which):
-        """which: "x" | "r" -> (max_iter, n) array; "scalars" -> (2, max_iter): rows a, b."""
+        """which: "x" | "r" -> (max_iter, n) array; "scalars" -> (2, max_iter): rows a, b.
+        After a tolerance stop at k: stop + 1 rows / columns."""
         sel = {"x": 0, "r": 1, "scalars": 2}[which]
         out = np.empty((2, self._max_iter)) if sel == 2 else np.empty((self._max_iter, self.n))
         _lib.check(self._lib.cgx_fetch_capture_host(self._ctx, sel, _lib.dptr(out)))
+        stop = self._stop()
+        if stop >= 0:
+            out = (out[:, :stop + 1] if sel == 2 else out[:stop + 1]).copy()
         return out
 
     def set_gv_replace(self, flags=None):
@@ -169,9 +204,14 @@ class Session:
         return dict(zip(("a", "a1", "b", "nu", "nu1", "mu", "eta", "delta", "gamma"), out.tolist()))
 
     def fetch(self, want_x=True, want_hist=True):
+        """x and the (4, max_iter) history rows; (4, stop + 1) after a tolerance stop."""
         x = np.empty(self.n) if want_x else None
         hist = np.empty((len(_lib.HIST_NAMES), self._max_iter)) if want_hist else None
         _lib.check(self._lib.cgx_fetch_host(self._ctx, _lib.dptr(x), _lib.dptr(hist)))
+        if hist is not None:
+            stop = self._stop()
+            if stop >= 0:
+                hist = hist[:, :stop + 1].copy()
         return x, hist
 
     def vector(self, name):
@@ -180,11 +220,15 @@ class Session:
         return out
 
     def solve(self, variant, b, x0, max_iter, x_true=None, histories=_lib.HIST_NAMES, path="auto",
-              return_x=True, x_out=None):
+              return_x=True, x_out=None, tol=None):
         """The reference call in one C-ABI round trip (host buffers in, host buffers out).
 
         ``x_out``: optional caller-owned (e.g. pinned) float64 array that receives x.
+        ``tol``: stop once nu_k <= tol^2 nu_0 (``set_tolerance``; None: the session's own); the
+        histories then hold ``info["stop_iter"] + 1`` entries.
         Returns (x, {history name: (max_iter,) array}, info)."""
+        if tol is not None:
+            _lib.check_tol(tol)
         b = _f64(b, self.n, "b")
         x0 = _f64(x0, self.n, "x0")
         xt = None if x_true is None else _f64(x_true, self.n, "x_true")
@@ -198,17 +242,13 @@ class Session:
             x = np.empty(self.n) if return_x else None
         hist = np.zeros((len(_lib.HIST_NAMES), int(max_iter))) if mask else None
         info = _lib.CgxInfo()
-        rc = self._lib.cgx_solve_host(self._ctx, _lib.VARIANT_IDS[variant], _lib.dptr(b), _lib.dptr(x0),
-                                      _lib.dptr(xt), self.n, int(max_iter), mask, _lib.PATHS[path],
-                                      _lib.dptr(x), _lib.dptr(hist), C.byref(info))
+        rc = self._with_tol(tol, lambda: self._lib.cgx_solve_host(
+            self._ctx, _lib.VARIANT_IDS[variant], _lib.dptr(b), _lib.dptr(x0), _lib.dptr(xt), self.n, int(max_iter),
+            mask, _lib.PATHS[path], _lib.dptr(x), _lib.dptr(hist), C.byref(info)))
         _lib.check(rc, allow_breakdown=True)
         self.info = info.as_dict()
         self._max_iter = int(max_iter)
-        out = {}
-        for i, name in enumerate(_lib.HIST_NAMES):
-            if name in histories and (xt is not None or "error" not in name):
-                out[name] = hist[i].copy()
-        return x, out, self.info
+        return x, _hist_dict(hist, histories, xt is not None, self.info["stop_iter"]), self.info
 
     # -- primitives (unit tests) -------------------------------------------------------
     def spmv(self, v):
@@ -225,7 +265,17 @@ class Session:
         return out.value
 
 
-def solve_batch(items, histories=_lib.HIST_NAMES, return_x=True):
+def _hist_dict(hist, histories, has_xt, stop):
+    """{name: row} of the selected histories, cut to stop + 1 entries after a tolerance stop."""
+    out = {}
+    end = stop + 1 if stop >= 0 else None
+    for i, name in enumerate(_lib.HIST_NAMES):
+        if name in histories and (has_xt or "error" not in name):
+            out[name] = hist[i][:end].copy()
+    return out
+
+
+def solve_batch(items, histories=_lib.HIST_NAMES, return_x=True, tol=None):
     """Independent solves side by side on one GPU, in ONE cooperative launch (cgx_batch_run).
 
     ``items``: sequence of ``(session, variant, b, x0, max_iter[, x_true])``, one distinct Session
@@ -233,7 +283,11 @@ def solve_batch(items, histories=_lib.HIST_NAMES, return_x=True):
     1/len(items) share of the SMs; its results are bitwise those of ``session.solve(...,
     path="persistent")`` with the same CTA shape (options ``pers_threads`` / ``pers_ctas``), and
     ``info["loop_ms"]`` is the duration of the shared launch.
+    ``tol``: one relative tolerance for every entry (None: each session's own); entries stop
+    independently, and each entry's histories are cut at its own ``info["stop_iter"]``.
     Returns ``[(x, {history name: (max_iter,) array}, info), ...]`` as ``Session.solve``."""
+    if tol is not None:
+        _lib.check_tol(tol)
     items = [tuple(it) for it in items]
     if not items:
         raise ValueError("solve_batch: no items")
@@ -257,18 +311,23 @@ def solve_batch(items, histories=_lib.HIST_NAMES, return_x=True):
     variants = np.array([_lib.VARIANT_IDS[it[1]] for it in items], dtype=np.int32)
     iters = np.array([int(it[4]) for it in items], dtype=np.int32)
     infos = (_lib.CgxInfo * count)()
-    rc = lib.cgx_batch_run(ctxs, count, _lib.iptr(variants), _lib.iptr(iters), mask, infos)
+    prev = [s._tol for s in sessions]
+    try:
+        if tol is not None:
+            for s in sessions:
+                s.set_tolerance(tol)
+        rc = lib.cgx_batch_run(ctxs, count, _lib.iptr(variants), _lib.iptr(iters), mask, infos)
+    finally:
+        if tol is not None:
+            for s, t in zip(sessions, prev):
+                s.set_tolerance(t)
     _lib.check(rc, allow_breakdown=True)
     results = []
     for sess, it, xt, info in zip(sessions, items, xts, infos):
         sess.info = info.as_dict()
         sess._max_iter = int(it[4])
         x, hist = sess.fetch(want_x=return_x, want_hist=bool(mask))
-        out = {}
-        for i, name in enumerate(_lib.HIST_NAMES):
-            if name in histories and (xt is not None or "error" not in name):
-                out[name] = hist[i].copy()
-        results.append((x, out, sess.info))
+        results.append((x, _hist_dict(hist, histories, xt is not None, -1) if mask else {}, sess.info))
     return results
 
 
