@@ -155,7 +155,8 @@ int cgx_get_scalars(cgx_ctx* ctx, double* out9);
  *      "stub_allreduce" = 1 replaces the multi-GPU scalar
  *      exchange by a local stand-in (timing experiment: exposed allreduce time). */
 int cgx_set_option(cgx_ctx* ctx, const char* name, int value);
-/* ---- stop at a relative tolerance (single-GPU contexts: stream path, persistent path, cgx_batch_run).
+/* ---- stop at a relative tolerance (one GPU: stream path, persistent path, cgx_batch_run; a partition:
+ *      z-slabs or a CSR row partition, stream path, and the persistent path on slabs).
  *      rtol = 0 (the default) switches it off: every run then does max_iter - 1 iterations.
  *      Otherwise 0 < rtol < 1 (anything else, NaN included, is CGX_ERR_ARG), and a run stops at
  *      stop_iter = the first k >= 1 with nu_k <= rtol^2 * nu_0, where nu_k = r~_k . r_k is the
@@ -169,8 +170,15 @@ int cgx_set_option(cgx_ctx* ctx, const char* name, int value);
  *      (and cgx_advance_stages) after the stop do nothing and return CGX_OK.  A breakdown is reported
  *      as before; a NaN nu never meets the tolerance.
  *      Takes effect at the next cgx_begin / cgx_run / cgx_solve_host / cgx_batch_run (per context).
- *      cgx_begin / cgx_group_begin refuse a rank of a partition with a tolerance set
- *      (CGX_ERR_UNSUPPORTED); set 0 to run it. */
+ *      Partitions: the call is collective -- every rank sets the same rtol.  nu_k is then the all-rank
+ *      total, the same bits on every rank, so every rank stops at the same stop_iter; the contract above
+ *      holds per rank against the same partition (same world, path and options) run without a
+ *      tolerance and with max_iter = stop_iter + 1 (not against one GPU, which a partition matches only
+ *      to rounding).  Refused with CGX_ERR_UNSUPPORTED before anything is enqueued: ranks of one
+ *      cgx_group_begin whose tolerances differ; a scalar exchange other than peer to peer (NCCL, or the
+ *      stub_allreduce stand-in, under which the ranks' nu differ); and cgx_begin / cgx_run /
+ *      cgx_solve_host on a single rank whose peers are contexts of this process (cgx_dist_attach_ctx:
+ *      drive those with cgx_group_*).  Ranks attached through CUDA IPC run with cgx_begin as usual. */
 int cgx_set_tolerance(cgx_ctx* ctx, double rtol);
 /* timing experiments: 16 %globaltimer stamps written by the last vector pass under
  * cgx_set_option("debug_skip", 2): [0] kernel start, [1] scalars folded, [2] CTA 0 done (ns). */

@@ -6,6 +6,12 @@ un-preconditioned, x0 = 0, exactly `max_iter` loop trips (`for k in range(max_it
 hs_cg.py:36, pr_cg.py:49), no convergence test, no history; `times` is a dict with the wall
 time under 'tot' on rank 0 and None elsewhere (hs_cg.py:13-16,66).
 
+An extension: `solve_to_tol("pr_cg", comm, A, b, max_iter, tol)` (any of the five names) stops every
+rank at the first k >= 1 with nu_k <= tol^2 nu_0 (nu_k = ||r_k||^2 here, the all-rank total;
+include/cgx.h cgx_set_tolerance), and rank 0's `times` then also holds 'stop_iter' (-1 when `max_iter`
+trips ran first).  Every rank must pass the same `tol`.  The five solvers keep the reference's signature
+and outputs.
+
 Here `comm` is a `GpuComm` (one rank per GPU; `Get_size/Get_rank/Barrier` as mpi4py's) -- or
 anything with those three methods, e.g. a real `MPI.COMM_WORLD` -- and the rows are
 partitioned in contiguous blocks as in the reference (rank r owns rows r*m .. (r+1)*m-1).
@@ -27,6 +33,7 @@ import time
 import numpy as np
 import scipy.sparse as sps
 
+from . import _lib
 from .operators import PoissonStencil
 from .session import Session
 
@@ -112,8 +119,10 @@ def _operator_session(comm, A, m):
     return sess
 
 
-def _run(tag, comm, A, b, max_iter):
+def _run(tag, comm, A, b, max_iter, tol=None):
     size, rank = comm.Get_size(), comm.Get_rank()
+    if tol is not None:
+        _lib.check_tol(tol)
     b = np.ascontiguousarray(np.asarray(b, dtype=np.float64))
     m = len(b)
     times = {'tot': 0., 'c_ip': 0., 'c_mv': 0., 'w_mv': 0., 'w_ip': 0., 'w_vec': 0.} if rank == 0 else None
@@ -125,10 +134,12 @@ def _run(tag, comm, A, b, max_iter):
         sess.load_problem_local(b, x0, None)
     comm.Barrier()                                     # hs_cg.py:30-33: timing starts after a barrier
     t0 = time.perf_counter()
-    sess.run(tag, int(max_iter) + 1, histories=())
+    info = sess.run(tag, int(max_iter) + 1, histories=(), tol=tol)
     comm.Barrier()
     if rank == 0:
         times['tot'] += time.perf_counter() - t0
+        if tol is not None:
+            times['stop_iter'] = int(info["stop_iter"])
     x = sess.fetch(want_hist=False)[0] if size == 1 else sess.fetch_local(want_hist=False)[0]
     return x, times
 
@@ -151,6 +162,20 @@ def pr_cg(comm, A, b, max_iter):
 
 def pipe_pr_cg(comm, A, b, max_iter):
     return _run("pipe_pr", comm, A, b, max_iter)
+
+
+SOLVERS = {"hs_cg": "hs", "cg_cg": "cg", "gv_cg": "gv", "pr_cg": "pr", "pipe_pr_cg": "pipe_pr"}
+
+
+def solve_to_tol(name, comm, A, b, max_iter, tol):
+    """`name(comm, A, b, max_iter)` (a key of SOLVERS) that stops every rank at the first k >= 1 with
+    nu_k <= tol^2 nu_0; rank 0's `times` also holds 'stop_iter'.  The five solvers keep the reference's
+    exact signature."""
+    if name not in SOLVERS:
+        raise ValueError(f"unknown solver {name!r}; one of {sorted(SOLVERS)}")
+    if tol is None:
+        raise ValueError("tol is required (the solvers themselves run max_iter trips)")
+    return _run(SOLVERS[name], comm, A, b, max_iter, tol)
 
 
 def model_problem(n, kappa=1e6, rho=0.9):

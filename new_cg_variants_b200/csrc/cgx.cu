@@ -570,6 +570,7 @@ void launch_instrument(cgx_ctx* c, Args g) {
 void launch_hist_consume(cgx_ctx* c, Args g) {
   if (c->dist.world <= 1) return;
   g.d = c->dist;
+  g.scpar = c->scpar;                 // (its stop test)
   g.pend_e[0] = c->epoch;
   if (c->dist.mode == 2) cudaStreamWaitEvent(c->stream, c->ev_red[c->epoch % kSlots], 0);
   hist_consume_kernel<<<1, 32, 0, c->stream>>>(g);
@@ -863,9 +864,6 @@ static int begin_prepare(cgx_ctx* c, int variant, int max_iter, unsigned hist_ma
     return fail(CGX_ERR_ARG, "cgx_begin: unknown path %d", path);
   if (c->dist.world > 1 && !c->dist_ready)
     return fail(CGX_ERR_ARG, "cgx_begin: cgx_dist_commit has not been called on this rank");
-  if (c->dist.world > 1 && c->tol > 0.0)
-    return fail(CGX_ERR_UNSUPPORTED, "cgx_begin: a tolerance stops single-GPU solves only (rank %d of a partition has one set)",
-                c->dist.rank);
   CU(cudaSetDevice(c->device));
   if (c->tol > 0.0 && !c->h_stop) {
     CU(cudaHostAlloc(&c->h_stop, 2 * sizeof(int), cudaHostAllocDefault));
@@ -971,10 +969,26 @@ static int check_device_flags(cgx_ctx* c, const char* who) {
 
 // Lockstep driver: `count` contexts (ranks of one partitioned problem, or a single context).
 static int group_begin(cgx_ctx** cs, int count, int variant, int max_iter, unsigned hist_mask, int path) {
-  for (int i = 0; i < count; ++i)       // (before any rank has enqueued anything)
-    if (cs[i] && cs[i]->dist.world > 1 && cs[i]->tol > 0.0)
-      return fail(CGX_ERR_UNSUPPORTED, "cgx_begin: a tolerance stops single-GPU solves only (rank %d of a partition has one set)",
-                  cs[i]->dist.rank);
+  // A tolerance on a partition (checked before any rank has enqueued anything).  Every rank must stop at
+  // the same k: they all test the same all-rank nu against the same threshold, so they must hold the same
+  // tolerance, exchange their records peer to peer (mode 1: in mode 3 the ranks' nu differ by construction;
+  // mode 2, NCCL, is not supported with a tolerance), and be driven either one process per rank or all
+  // together by cgx_group_* -- a lone rank whose peers are contexts of this process would leave them behind.
+  for (int i = 0; i < count; ++i) {
+    const cgx_ctx* c = cs[i];
+    if (!c || c->dist.world <= 1 || (c->tol <= 0.0 && cs[0]->tol <= 0.0)) continue;
+    if (c->tol != cs[0]->tol)
+      return fail(CGX_ERR_UNSUPPORTED, "cgx_begin: the ranks of a partition must set the same tolerance (rank %d: %g, rank %d: %g)",
+                  cs[0]->dist.rank, cs[0]->tol, c->dist.rank, c->tol);
+    if (c->dist.mode != 1)
+      return fail(CGX_ERR_UNSUPPORTED, "cgx_begin: a tolerance on a partition needs the peer-to-peer scalar exchange "
+                  "(rank %d uses %s)", c->dist.rank, c->dist.mode == 2 ? "NCCL" : "the stub_allreduce stand-in");
+    if (count == 1)
+      for (int r = 0; r < c->dist.world; ++r)
+        if (r != c->dist.rank && !c->peer_ipc[r])
+          return fail(CGX_ERR_UNSUPPORTED, "cgx_begin: rank %d of a partition with a tolerance has peers in this process: "
+                      "drive the partition with cgx_group_begin / cgx_group_advance", c->dist.rank);
+  }
   bool same_device = count > 1;
   for (int i = 1; i < count; ++i) same_device = same_device && cs[i]->device == cs[0]->device;
   for (int i = 0; i < count; ++i) {
@@ -1066,8 +1080,11 @@ static int group_advance(cgx_ctx** cs, int count, int niter) {
   } else {
     const int ns = iter_stage_count(c0);
     if (c0->cur_stage != 0) return fail(CGX_ERR_ARG, "cgx_advance: an iteration is half done (cgx_advance_stages); finish it first");
-    // with a tolerance (single contexts only): chunks of kTolChunk iterations, each followed by a copy of
-    // stop_k into pinned slot j & 1; chunk j is enqueued once chunk j - 2 has completed and did not stop
+    // with a tolerance: chunks of kTolChunk iterations, each followed by a copy of stop_k into pinned slot
+    // j & 1; chunk j is enqueued once chunk j - 2 has completed and did not stop.  On a partition every rank
+    // must enqueue the same launches (the host epoch counters become LL tags all ranks agree on): the word
+    // copied at the end of chunk j - 2 is the stop_k folded from the all-rank totals, the same bits on every
+    // rank, so independent processes make the same choice.  In a group, c0's word decides for all ranks.
     const bool poll = c0->run_tol > 0.0;
     const int first = c0->cur_k + 1;
     for (int k = first; k <= last; ++k) {

@@ -107,9 +107,12 @@ struct Args {
 };
 
 // Every kernel of the iteration loop starts with this test (after griddepcontrol.wait where the kernel
-// is launched with programmatic serialisation: stop_k is written by an earlier kernel).  g.sc->stop_k was
-// written before the launch, so every CTA takes the same branch.
-__device__ __forceinline__ bool after_stop(const Args& g) { return g.tol_on && past_stop(g.sc, g.k); }
+// is launched with programmatic serialisation: stop_k is written by an earlier kernel).  stop_k was
+// written before the launch, so every CTA takes the same branch.  On a partition the scalars live in
+// sc[scpar]: every consumer of pending records persists its fold there, also after the stop (dist_fold),
+// so the parity the host hands to a launch always holds the latest stop_k.  (One GPU: scpar = 0.)
+// The vector passes of a partition do not take this test at entry: they fold first (dist_fold).
+__device__ __forceinline__ bool after_stop(const Args& g) { return g.tol_on && past_stop(g.sc + g.scpar, g.k); }
 
 // An SpMV input vector: the owned slab and (multi-GPU) the ghost planes below and above.
 struct VecIn { const double* v; const double* lo; const double* hi; };
@@ -159,16 +162,15 @@ __device__ __forceinline__ double predict_beta(bool meurant, double nu, double a
 }
 
 // Scalar recurrences that close a fused reduction (run by one thread with the grid -- or,
-// multi-GPU, the all-rank -- totals).  kind: FK_* of cgx_common.cuh.  stop_test: look for the
-// tolerance stop (partitions, which refuse a tolerance, leave it out of their scalar fold).
-__device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc, const double* acc, int k,
-                                               bool stop_test = true) {
+// multi-GPU, the all-rank -- totals).  kind: FK_* of cgx_common.cuh.  The tolerance is tested where
+// nu_k is assigned (note_stop; without a tolerance thr is NaN and nothing stops).
+__device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc, const double* acc, int k) {
   if (kind == FK_HS_NU) {                    // hs_cg.py:120-121
     const double nu1 = sc->nu;
     sc->nu1 = nu1; sc->nu = acc[0];
     sc->b = div_(acc[0], nu1);
     note_breakdown(sc, k, sc->a, sc->b);
-    if (stop_test) note_stop(sc, k);
+    note_stop(sc, k);
   } else if (kind == FK_HS_MU) {             // hs_cg.py:124-125
     sc->mu = acc[0];
     sc->a1 = sc->a; sc->a = div_(sc->nu, acc[0]);
@@ -180,10 +182,10 @@ __device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc,
     sc->nu1 = nu1; sc->nu = nu; sc->eta = eta; sc->b = bb; sc->mu = mu;
     sc->a1 = a1; sc->a = div_(nu, mu);
     note_breakdown(sc, k, sc->a, bb);
-    if (stop_test) note_stop(sc, k);
+    note_stop(sc, k);
   } else if (kind == FK_PR_NU) {             // pr_cg.py:157 (consumed by the SpMV pass)
     sc->nu1 = sc->nu; sc->nu = acc[0];
-    if (stop_test) note_stop(sc, k);
+    note_stop(sc, k);
   } else if (kind == FK_PR_SP) {             // pr_cg.py:154-158 then :149-150
     const double mu = acc[0], del = acc[1], gam = acc[2], nu = sc->nu;
     sc->mu = mu; sc->del = del; sc->gam = gam;
@@ -198,7 +200,7 @@ __device__ __forceinline__ void apply_finalize(int kind, bool meurant, Scal* sc,
     sc->a1 = sc->a; sc->a = an;
     sc->b = predict_beta(meurant, nu, an, del, gam);
     note_breakdown(sc, k, an, sc->b);
-    if (stop_test) note_stop(sc, k);
+    note_stop(sc, k);
   }
 }
 
@@ -263,7 +265,14 @@ __device__ __forceinline__ void dist_totals(const Args& g, u64 e, int nr, double
 // Every CTA of a kernel that needs alpha/beta: fold the pending reductions into the scalars
 // (redundantly, identical bits everywhere); CTA 0 persists the result in the other parity.
 // dist_fold: the warp-0 part (call with threadIdx.x < 32); the caller synchronises the CTA (or
-// its compute warps) before reading sh_ab.
+// its compute warps) before reading sh_ab[0..2].
+// Tolerance stop: nu_k of a partition is known only here, in the first consumer of iteration k + 1 (HS:
+// in EW_HS2 of iteration k); apply_finalize makes the test where it assigns nu.  A record of an
+// iteration after stop_k was never published (its launch returned): it is skipped without a poll; the
+// records are in order, so once one sets stop_k the rest are skipped.
+// The fold is persisted also after the stop -- the parity the host flips to must hold the scalars -- and
+// is then exactly what the flush of a run ending at stop_k persists.
+// sh_ab[2] != 0: this launch belongs to an iteration after stop_k and must return without any work.
 __device__ __forceinline__ void dist_fold(const Args& g, bool meurant, double* sh_ab) {
   const bool stamp = (g.dbg & 2) && blockIdx.x == 0 && threadIdx.x == 0;
   {
@@ -288,7 +297,7 @@ __device__ __forceinline__ void dist_fold(const Args& g, bool meurant, double* s
     if (stamp) g.dbg_t[4] = (u64)clock64();
 #pragma unroll
     for (int q = 0; q < 3; ++q) {
-      if (q < g.npend) {
+      if (q < g.npend && !(g.tol_on && past_stop(&s, g.pend_k[q]))) {
         double acc[kNRed];
         if (ll) {
           const double v = on[q] ? ll_finish(rq[q], g.pend_e[q], &w->error) : 0.0;
@@ -302,12 +311,13 @@ __device__ __forceinline__ void dist_fold(const Args& g, bool meurant, double* s
           dist_totals(g, g.pend_e[q], fk_width(g.pend_kind[q]), acc);
         }
         if (stamp) g.dbg_t[5 + 2 * q] = (u64)clock64();
-        apply_finalize(g.pend_kind[q], meurant, &s, acc, g.pend_k[q], false);
+        apply_finalize(g.pend_kind[q], meurant, &s, acc, g.pend_k[q]);
         if (stamp) g.dbg_t[6 + 2 * q] = (u64)clock64();
       }
     }
     if (threadIdx.x == 0) {
       sh_ab[0] = s.a; sh_ab[1] = s.b;
+      sh_ab[2] = (g.tol_on && past_stop(&s, g.k)) ? 1.0 : 0.0;
       if (blockIdx.x == 0 && g.npend) {          // (tmp[] is initialisation scratch: not carried over)
         Scal* o = &g.sc[g.scpar ^ 1];
         o->a = s.a; o->a1 = s.a1; o->b = s.b; o->nu = s.nu; o->nu1 = s.nu1; o->mu = s.mu; o->eta = s.eta;
@@ -317,11 +327,13 @@ __device__ __forceinline__ void dist_fold(const Args& g, bool meurant, double* s
   }
   if (stamp) g.dbg_t[9] = (u64)clock64();
 }
-__device__ __forceinline__ void dist_scalars(const Args& g, bool meurant, double& a, double& b) {
-  __shared__ double sh_ab[2];
+// (returns true when the launch belongs to an iteration after a tolerance stop: see dist_fold)
+__device__ __forceinline__ bool dist_scalars(const Args& g, bool meurant, double& a, double& b) {
+  __shared__ double sh_ab[3];
   if (threadIdx.x < 32) dist_fold(g, meurant, sh_ab);
   __syncthreads();
   a = sh_ab[0]; b = sh_ab[1];
+  return sh_ab[2] != 0.0;
 }
 
 // The SpMV-input vector a vector pass produces: also store its first / last plane into the
@@ -558,7 +570,7 @@ __global__ void __launch_bounds__(kBlock) ew_kernel(const Args g) {
   const bool stamp = (g.dbg & 2) && blockIdx.x == 0 && threadIdx.x == 0;
   pdl_launch_dependents();
   pdl_wait();                          // nothing of the previous kernel's data is touched before this
-  if (after_stop(g)) return;
+  if (!dist && after_stop(g)) return;  // (a partition decides after its fold, below)
   if (stamp) g.dbg_t[0] = (u64)clock64();
   if (dist) {
     const i64 rot0 = (g.hout_n > 0 && g.d.has_hi) ? nv - (g.d.plane >> 1) : 0;
@@ -568,7 +580,7 @@ __global__ void __launch_bounds__(kBlock) ew_kernel(const Args g) {
     // warps 1..7 prefetch while warp 0 folds the records (its own prefetch follows its loads, so
     // the few record loads are not queued behind the prefetch burst)
     if (pf && threadIdx.x >= 32) ew_prefetch<KID, PM>(g, 2 * i0);
-    dist_scalars(g, MEURANT, a, b);
+    if (dist_scalars(g, MEURANT, a, b)) return;     // folded and persisted: nothing of this iteration runs
     if (pf && threadIdx.x < 32) ew_prefetch<KID, PM>(g, 2 * i0);
   } else { a = g.sc->a; b = g.sc->b; }
   if (stamp) g.dbg_t[1] = (u64)clock64();
@@ -996,6 +1008,7 @@ __global__ void __launch_bounds__(kBlock) instrument_kernel(const Op A, const Ar
 
 // multi-GPU: fold all ranks' instrumentation records of epoch pend_e[0] into history entry k
 static __global__ void hist_consume_kernel(const Args g) {
+  if (after_stop(g)) return;           // (its record was never published)
   double acc[kNRed];
   dist_totals(g, g.pend_e[0], 4, acc);
   if (threadIdx.x == 0) {
@@ -1014,6 +1027,7 @@ static __global__ void flush_scalars_kernel(const Args g) {
 // multi-GPU: copy the first / last plane of v into the neighbours' ghost planes of channel
 // hout_ch (initialisation SpMVs, instrumentation x, x_true) and publish the halo epoch.
 static __global__ void __launch_bounds__(kBlock) halo_push_kernel(const Args g, const double* __restrict__ v) {
+  if (after_stop(g)) return;
   const i64 pl = g.d.plane;
   const i64 stride = (i64)gridDim.x * kBlock;
   for (i64 i = (i64)blockIdx.x * kBlock + threadIdx.x; i < pl; i += stride) {
@@ -1026,6 +1040,7 @@ static __global__ void __launch_bounds__(kBlock) halo_push_kernel(const Args g, 
 // CSR row partition: gather the entries of v the other ranks need and store them into their staging
 // arrays (channel hout_ch, parity hout_par), then publish the epoch to every destination.
 static __global__ void __launch_bounds__(kBlock) csr_halo_push_kernel(const Args g, const double* __restrict__ v) {
+  if (after_stop(g)) return;
   const int total = g.d.send_ptr[g.d.world];
   const i64 stride = (i64)gridDim.x * kBlock;
   for (i64 i = (i64)blockIdx.x * kBlock + threadIdx.x; i < total; i += stride) {
@@ -1136,6 +1151,7 @@ static __global__ void init_scalars_kernel(const Args g, int variant_class, int 
   sc->b = 0.0;
   sc->breakdown = -1;
   sc->stop_k = -1;
+  g.sc[g.scpar ^ 1].stop_k = -1;       // (a partition's other parity: no stale stop of an earlier run)
   sc->thr = tol > 0.0 ? mul_(mul_(tol, tol), nu) : nan("");
   if (variant_class == 2) sc->b = predict_beta(meurant != 0, nu, sc->a, sc->del, sc->gam);
   note_breakdown(sc, 0, sc->a, sc->b);

@@ -477,6 +477,10 @@ __device__ __forceinline__ void persistent_body(const PersRank<Op>& pr, const Pe
     double red[kPersRed];
     // ---- vector stage(s) ----------------------------------------------------------
     fold_pending();
+    // partition: nu of iteration k - 1 (all but HS) is known only now, from the records of k - 1.  After
+    // a stop there, every CTA of every rank folded the same totals: all leave before any work or sync
+    // point of iteration k, so the epoch counters stay those of a run ending at stop_k
+    if (dist && s.stop_k >= 0 && k > s.stop_k) break;
 #pragma unroll
     for (int j = 0; j < kPersRed; ++j) red[j] = 0.0;
     {

@@ -69,7 +69,7 @@ pr_fused_kernel(const __grid_constant__ CUtensorMap tm_p, const __grid_constant_
   if (g.tol_on) {                      // stop_k is visible only after the wait: no prologue overlap then
     pdl_launch_dependents();
     pdl_wait();
-    if (after_stop(g)) return;
+    if (!DIST && after_stop(g)) return;   // (a partition decides after its fold, below)
   }
   if (tid == 0) {
 #pragma unroll
@@ -82,13 +82,19 @@ pr_fused_kernel(const __grid_constant__ CUtensorMap tm_p, const __grid_constant_
 
   double a, b;
   if constexpr (DIST) {
-    // only the compute warps need the scalars: the producer warp starts its copies at once
-    __shared__ double sh_ab[2];
+    // only the compute warps need the scalars: the producer warp starts its copies at once -- except
+    // with a tolerance, where the fold decides whether this iteration runs at all (dist_fold): every
+    // thread waits for it, so that no copy is issued, and none is left in flight, by a launch that returns
+    __shared__ double sh_ab[3];
     if (tid < kFConsumers) {
       if (tid < 32) dist_fold(g, MEUR, sh_ab);
       named_bar_sync(1, kFConsumers);
       a = sh_ab[0]; b = sh_ab[1];
     } else { a = b = 0.0; }
+    if (g.tol_on) {                    // (the fold wrote sh_ab[2] before the compute warps' barrier)
+      __syncthreads();
+      if (sh_ab[2] != 0.0) return;
+    }
   } else { a = g.sc->a; b = g.sc->b; }
   const double ds = g.dinv_s;
   auto M = [&](double v) { return PM == 2 ? mul_(ds, v) : v; };

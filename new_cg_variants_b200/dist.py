@@ -225,6 +225,11 @@ class _RankBase:
     def set_option(self, name, value):
         _lib.check(self._lib.cgx_set_option(self._ctx, name.encode(), int(value)))
 
+    def _set_tol(self, tol):
+        """This rank's relative tolerance for the next begin / run (None or 0: off).  Collective in
+        effect: every rank of a partition must set the same value (include/cgx.h cgx_set_tolerance)."""
+        _lib.check(self._lib.cgx_set_tolerance(self._ctx, 0.0 if tol is None else _lib.check_tol(tol)))
+
     def set_profile(self, on=True):
         _lib.check(self._lib.cgx_set_profile(self._ctx, 1 if on else 0))
 
@@ -303,7 +308,12 @@ class DistSession(_RankBase):
         _lib.check(self._lib.cgx_load_problem_host(self._ctx, _lib.dptr(b), _lib.dptr(x0),
                                                    _lib.dptr(x_true), self.n))
 
-    def run(self, variant, max_iter, histories=(), path="auto"):
+    def run(self, variant, max_iter, histories=(), path="auto", tol=None):
+        """``tol``: stop every rank at the first k >= 1 with nu_k <= tol^2 nu_0 (nu: the all-rank total,
+        so every rank stops at the same ``info["stop_iter"]``); every rank must pass the same value."""
+        if tol is not None:
+            _lib.check_tol(tol)
+        self._set_tol(tol)
         info = _lib.CgxInfo()
         p = _lib.PATHS[path]
         rc = self._lib.cgx_run(self._ctx, _lib.VARIANT_IDS[variant], int(max_iter), _mask(histories), p,
@@ -314,8 +324,12 @@ class DistSession(_RankBase):
         return self.info
 
     def solve_local(self, variant, b_loc, x0_loc, max_iter, x_true_loc=None, histories=(), return_x=True,
-                    path="auto", x_out=None):
-        """The C-ABI round trip with this rank's HOST slices (cgx_solve_host)."""
+                    path="auto", x_out=None, tol=None):
+        """The C-ABI round trip with this rank's HOST slices (cgx_solve_host).  ``tol`` as in ``run``;
+        the histories then hold ``info["stop_iter"] + 1`` entries."""
+        if tol is not None:
+            _lib.check_tol(tol)
+        self._set_tol(tol)
         mask = _mask(histories)
         x = x_out if x_out is not None else (np.empty(self.n) if return_x else None)
         hist = np.zeros((len(_lib.HIST_NAMES), int(max_iter))) if mask else None
@@ -326,15 +340,20 @@ class DistSession(_RankBase):
         _lib.check(rc, allow_breakdown=True)
         self.info = info.as_dict()
         self._max_iter = int(max_iter)
+        stop = self.info["stop_iter"]
+        end = stop + 1 if stop >= 0 else None
         out = {}
         for i, name in enumerate(_lib.HIST_NAMES):
             if name in histories and (x_true_loc is not None or "error" not in name):
-                out[name] = hist[i].copy()
+                out[name] = hist[i][:end].copy()
         return x, out, self.info
 
-    def solve(self, variant, b, x0, max_iter, x_true=None, histories=_lib.HIST_NAMES, return_x=True, path="auto"):
+    def solve(self, variant, b, x0, max_iter, x_true=None, histories=_lib.HIST_NAMES, return_x=True, path="auto",
+              tol=None):
+        if tol is not None:
+            _lib.check_tol(tol)
         return self.solve_local(variant, self.local(b), self.local(x0), max_iter, self.local(x_true),
-                                histories, return_x, path)
+                                histories, return_x, path, tol=tol)
 
     def gather_x(self, x_local):
         """Global x on every rank (host side, through torch.distributed objects)."""
@@ -415,7 +434,13 @@ class GroupSession:
             _lib.check(self._lib.cgx_group_load_problem_host(self._arr, self.world, _lib.dptr(b), _lib.dptr(x0),
                                                              _lib.dptr(xt), self.n))
 
-    def begin(self, variant, max_iter, histories=(), path="stream"):
+    def begin(self, variant, max_iter, histories=(), path="stream", tol=None):
+        """``tol``: stop all ranks at the first k >= 1 with nu_k <= tol^2 nu_0 (nu: the all-rank total);
+        ``advance`` after the stop does nothing.  None: no tolerance."""
+        if tol is not None:
+            _lib.check_tol(tol)
+        for m in self.members:
+            m._set_tol(tol)
         if self.world == 1:
             _lib.check(self._lib.cgx_begin(self.members[0]._ctx, _lib.VARIANT_IDS[variant], int(max_iter),
                                            _mask(histories), _lib.PATHS[path]))
@@ -432,10 +457,13 @@ class GroupSession:
         else:
             _lib.check(self._lib.cgx_group_advance(self._arr, self.world, int(niter)))
 
-    def solve(self, variant, b, x0, max_iter, x_true=None, histories=_lib.HIST_NAMES, path="stream"):
-        """-> (global x, {history: array}, [per-rank info])."""
+    def solve(self, variant, b, x0, max_iter, x_true=None, histories=_lib.HIST_NAMES, path="stream", tol=None):
+        """-> (global x, {history: array}, [per-rank info]).  ``tol`` as in ``begin``: the histories then
+        hold ``info["stop_iter"] + 1`` entries."""
+        if tol is not None:
+            _lib.check_tol(tol)
         self.load_problem(b, x0, x_true)
-        self.begin(variant, max_iter, histories, path)
+        self.begin(variant, max_iter, histories, path, tol=tol)
         self.advance(max_iter - 1)
         xs, hists = [], []
         for m in self.members:
@@ -445,11 +473,14 @@ class GroupSession:
         for h in hists[1:]:          # every rank holds the same global histories, bit for bit
             if not np.array_equal(h, hists[0]):
                 raise AssertionError("ranks disagree on the histories")
+        infos = [m.get_info() for m in self.members]
+        stop = infos[0]["stop_iter"]
+        end = stop + 1 if stop >= 0 else None
         out = {}
         for i, name in enumerate(_lib.HIST_NAMES):
             if name in histories and (x_true is not None or "error" not in name):
-                out[name] = hists[0][i].copy()
-        return np.concatenate(xs), out, [m.get_info() for m in self.members]
+                out[name] = hists[0][i][:end].copy()
+        return np.concatenate(xs), out, infos
 
 
 CsrDistSession = DistSession      # (a DistSession given a matrix instead of a PoissonStencil)
