@@ -110,6 +110,19 @@ int cgx_set_csr_host(cgx_ctx* ctx, int64_t n, int64_t nnz, const int32_t* indptr
  * (SURVEY.md section 8d; matrices/poisson_ca.mtx is the 16x16 instance). */
 int cgx_set_stencil(cgx_ctx* ctx, int dim, int64_t nx, int64_t ny, int64_t nz, double diag,
                     double off);
+/* Matrix-free symmetric variable-coefficient stencil, same ordering and grid shapes as
+ * cgx_set_stencil (dim 2: nz == 1 and cz == NULL; dim 3: cz required).  Host arrays of n
+ * doubles: diag[i] = A[i,i], cx[i] = A[i,i+1], cy[i] = A[i,i+nx], cz[i] = A[i,i+nx*ny]; the
+ * backward couplings follow by symmetry (A[i,i-1] = cx[i-1], ...).  A coupling that leaves the
+ * grid (cx at x = nx-1, cy at y = ny-1, cz at z = nz-1) must be 0.  Row sums visit the full
+ * 5/7-point pattern in canonical CSR order, zero couplings inside the grid included, so every
+ * product equals scipy's on the CSR matrix that stores that pattern.
+ * CGX_ERR_ARG: bad shape, NULL array, non-finite value or non-zero coupling off the grid.
+ * CGX_ERR_UNSUPPORTED: the grid exceeds int32 indexing, or ctx is a rank of a partition.
+ * Not accepted by cgx_batch_run (CGX_ERR_UNSUPPORTED); "tma" = 0 forces the generic kernel. */
+int cgx_set_stencil_coef_host(cgx_ctx* ctx, int dim, int64_t nx, int64_t ny, int64_t nz,
+                              const double* diag, const double* cx, const double* cy,
+                              const double* cz);
 
 /* ---- preconditioner.  Replaces the callable `preconditioner(v)` of the *_pcg solvers
  *      (figure_gen.py:40-44): dinv_host == NULL -> identity, else z = dinv * v
@@ -297,7 +310,8 @@ int cgx_group_advance(cgx_ctx** ctxs, int count, int niter);
  *      Returns CGX_ERR_BREAKDOWN if any entry broke down (infos[i].breakdown_iter tells which).
  *      CGX_ERR_ARG: count < 1, a NULL pointer, a bad variant or max_iter, a context listed twice.
  *      CGX_ERR_UNSUPPORTED, before anything is launched: entries on different devices, a rank of
- *      a partition, mixed operator kinds (CSR / stencil) or preconditioner modes (none / Jacobi
+ *      a partition, a variable-coefficient stencil (cgx_set_stencil_coef_host), mixed operator
+ *      kinds (CSR / stencil) or preconditioner modes (none / Jacobi
  *      vector / constant diagonal), a capture, a GV replacement schedule or "gv_manual" set, an
  *      entry that does not fit its share of the SMs, or a grid that is not co-resident.  After a
  *      refusal every context still runs normally with cgx_run. */

@@ -7,7 +7,7 @@ tchen-research/new_cg_variants on NVIDIA B200 (sm_100a).
 keep the reference's Python signatures; the arithmetic runs in ``libcgx_b200.so``
 (hand-written CUDA behind the C ABI of ``include/cgx.h``).  No CPU fallback.
 """
-from .operators import PoissonStencil, canonical_csr, poisson2d, poisson3d   # noqa: F401
+from .operators import PoissonStencil, VariableStencil, canonical_csr, poisson2d, poisson3d   # noqa: F401
 from .session import Session                                                  # noqa: F401
 from . import callbacks, cg_variants, cg_variants_mpi4py, experiments              # noqa: F401
 

@@ -52,6 +52,8 @@ PROTOTYPES = {
     "cgx_ctx_destroy": (C.c_int, [_P]),
     "cgx_set_csr_host": (C.c_int, [_P, C.c_int64, C.c_int64, c_int32_p, c_int32_p, c_double_p]),
     "cgx_set_stencil": (C.c_int, [_P, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_double]),
+    "cgx_set_stencil_coef_host": (C.c_int, [_P, C.c_int, C.c_int64, C.c_int64, C.c_int64, c_double_p, c_double_p,
+                                            c_double_p, c_double_p]),
     "cgx_set_jacobi_host": (C.c_int, [_P, c_double_p, C.c_int64]),
     "cgx_load_problem_host": (C.c_int, [_P, c_double_p, c_double_p, c_double_p, C.c_int64]),
     "cgx_load_problem_dev": (C.c_int, [_P, _P, _P, _P, C.c_int64]),

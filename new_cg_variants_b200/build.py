@@ -30,7 +30,7 @@ UNITS = [
     ("cgx_iter_pm1", "cgx_iter.cu", ["-DCGX_PM=1"]),
     ("cgx_iter_pm2", "cgx_iter.cu", ["-DCGX_PM=2"]),
     *[(f"cgx_pers_{nm}_pm{pm}", "cgx_pers.cu", [f"-DCGX_PERS_OP={op}", f"-DCGX_PERS_PM={pm}"])
-      for op, nm in ((2, "sten"), (1, "csr")) for pm in (0, 1, 2)],
+      for op, nm in ((2, "sten"), (1, "csr"), (3, "var")) for pm in (0, 1, 2)],
     ("cgx_fused", "cgx_fused.cu", []),
     ("cgx", "cgx.cu", []),
 ]

@@ -11,7 +11,7 @@ host every iteration against the device state (the replacement ``w = A r`` itsel
 the GPU).
 
 Every iteration runs in libcgx_b200 on the GPU (there is no CPU solve path).  ``A`` may be
-a scipy sparse matrix, a dense ndarray, or a ``PoissonStencil``.  ``preconditioner`` stays an
+a scipy sparse matrix, a dense ndarray, a ``PoissonStencil`` or a ``VariableStencil``.  ``preconditioner`` stays an
 opaque callable as in the reference; it is probed once and must act as a fixed diagonal
 scaling (identity or Jacobi, figure_gen.py:40-44), otherwise ``NotImplementedError``.
 
@@ -35,7 +35,7 @@ import scipy.sparse as sps
 from .. import _lib
 from .. import callbacks as _cbk
 from ..callbacks import CAPTURE_CALLBACKS, DEVICE_HISTORIES
-from ..operators import PoissonStencil, canonical_csr
+from ..operators import PoissonStencil, VariableStencil, canonical_csr
 from ..session import Session
 
 _OWN_KEYS = ("device", "path", "session", "return_info", "w_replace", "tol")
@@ -74,6 +74,8 @@ _CACHE_SIZE = 2
 def _fingerprint(A):
     if isinstance(A, PoissonStencil):
         return ("stencil", A.dim, A.nx, A.ny, A.nz, A.diag, A.off)
+    if isinstance(A, VariableStencil):         # (matched on identity, as a sparse matrix: the shape does not say which)
+        return ("varstencil", A.dim, A.nx, A.ny, A.nz)
     if sps.issparse(A):
         if A.format not in ("csr", "csc", "coo", "bsr", "dia"):
             A = A.tocsr()                      # e.g. LIL keeps object-dtype rows
@@ -154,7 +156,7 @@ def _ensure_x_true(A, b, extra, needed):
     if not needed or "x_true" in extra:
         return
     import scipy.sparse.linalg as spla
-    if isinstance(A, PoissonStencil):
+    if isinstance(A, (PoissonStencil, VariableStencil)):
         A = A.tocsr()
     solver = spla.spsolve if sps.issparse(A) else np.linalg.solve
     extra["x_true"] = solver(A.astype(np.double), np.asarray(b, dtype=np.double))
@@ -182,7 +184,7 @@ def _solve(name, tag, A, b, x0, max_iter, preconditioner, callbacks, kwargs):
     plan = _plan_w_replace(w_replace, max_iter) if tag == "gv" else None
     capture, other = _split_capture(generic)
     if not other and not isinstance(plan, str):
-        if capture and isinstance(A, PoissonStencil):
+        if capture and isinstance(A, (PoissonStencil, VariableStencil)):
             A = A.tocsr()                      # the callback bodies multiply / factor A on the host
         sess.set_gv_replace(plan)
         names = {cb.__name__ for cb in capture}
@@ -365,6 +367,8 @@ def solve_concurrently(methods, A, b, x0, max_iter, preconditioner=lambda x: x, 
     single-method functions; every method stops on its own)."""
     from ..session import solve_batch
     methods = list(methods)
+    if isinstance(A, VariableStencil):
+        raise NotImplementedError("solve_concurrently: a VariableStencil runs one solve per launch (call the solvers one by one)")
     for key in ("path", "w_replace", "session"):
         if key in kwargs:
             raise NotImplementedError(f"solve_concurrently: `{key}=` is not supported (persistent batch only)")

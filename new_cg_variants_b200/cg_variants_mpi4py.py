@@ -34,7 +34,7 @@ import numpy as np
 import scipy.sparse as sps
 
 from . import _lib
-from .operators import PoissonStencil
+from .operators import PoissonStencil, VariableStencil
 from .session import Session
 
 
@@ -120,6 +120,8 @@ def _operator_session(comm, A, m):
 
 
 def _run(tag, comm, A, b, max_iter, tol=None):
+    if isinstance(A, VariableStencil):
+        raise NotImplementedError("cg_variants_mpi4py: a VariableStencil runs on one GPU (Session, cg_variants)")
     size, rank = comm.Get_size(), comm.Get_rank()
     if tol is not None:
         _lib.check_tol(tol)

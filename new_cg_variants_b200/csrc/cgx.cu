@@ -67,6 +67,9 @@ static void free_op(cgx_ctx* c) {
   c->n_rowblk_b = 0;
   c->n_rowblk = 0;
   c->h_ptr.clear();
+  for (auto& q : c->d_coef) { cudaFree(q); q = nullptr; }
+  c->vsten = VarStencilOp{};
+  c->coef_tmap_ok = false;
   c->op_kind = 0;
 }
 static void free_problem(cgx_ctx* c) {
@@ -131,7 +134,7 @@ extern "C" int cgx_ctx_create(int device, cgx_ctx** out) {
   CU(cudaMemset(c->d_dbg_t, 0, sizeof(u64) * 16));
   CU(cudaMalloc(&c->d_pout, sizeof(PersOut)));
   CU(cudaMemset(c->d_pout, 0, sizeof(PersOut)));
-  CU(cudaMalloc(&c->d_prank, std::max(sizeof(PersRank<CsrOp>), sizeof(PersRank<StencilOp>)) * kMaxWorld));
+  CU(cudaMalloc(&c->d_prank, std::max({sizeof(PersRank<CsrOp>), sizeof(PersRank<StencilOp>), sizeof(PersRank<VarStencilOp>)}) * kMaxWorld));
   c->dist.world = 1;
   *out = c;
   return CGX_OK;
@@ -318,6 +321,52 @@ extern "C" int cgx_set_stencil(cgx_ctx* c, int dim, int64_t nx, int64_t ny, int6
   return set_stencil(c, dim, nx, ny, nz, diag, off, 0, 0);
 }
 
+// A coupling that leaves the grid must be 0: cx at x = nx-1, cy at y = ny-1, cz at z = nz-1.
+static const char* coef_check(i64 nx, i64 ny, i64 nz, const double* diag, const double* cx, const double* cy,
+                              const double* cz) {
+  const i64 plane = nx * ny, n = plane * nz;
+  for (i64 i = 0; i < n; ++i) {
+    if (!std::isfinite(diag[i]) || !std::isfinite(cx[i]) || !std::isfinite(cy[i]) || (cz && !std::isfinite(cz[i])))
+      return "a coefficient is not finite";
+    const i64 x = i % nx, y = (i / nx) % ny, z = i / plane;
+    if ((x == nx - 1 && cx[i] != 0.0) || (y == ny - 1 && cy[i] != 0.0) || (cz && z == nz - 1 && cz[i] != 0.0))
+      return "a coupling that leaves the grid is not 0";
+  }
+  return nullptr;
+}
+
+extern "C" int cgx_set_stencil_coef_host(cgx_ctx* c, int dim, int64_t nx, int64_t ny, int64_t nz, const double* diag,
+                                         const double* cx, const double* cy, const double* cz) {
+  if (!c || (dim != 2 && dim != 3) || nx < 1 || ny < 1 || nz < 1 || (dim == 2 && (nz != 1 || cz)) || (dim == 3 && !cz) ||
+      !diag || !cx || !cy)
+    return fail(CGX_ERR_ARG, "cgx_set_stencil_coef_host: bad arguments (dim 2: nz == 1 and no cz; dim 3: cz required)");
+  if (c->dist.world > 1)
+    return fail(CGX_ERR_UNSUPPORTED, "cgx_set_stencil_coef_host: this context is a rank of a partitioned run; "
+                "variable-coefficient stencils run on one GPU");
+  const i64 n = nx * ny * nz;
+  if (n + 2 * nx * ny >= (1ll << 31))
+    return fail(CGX_ERR_UNSUPPORTED, "cgx_set_stencil_coef_host: grid too large for int32 indexing");
+  if (const char* why = coef_check(nx, ny, nz, diag, cx, cy, cz)) return fail(CGX_ERR_ARG, "cgx_set_stencil_coef_host: %s", why);
+  CU(cudaSetDevice(c->device));
+  free_op(c);
+  reset_size(c, n);
+  const double* src[4] = {diag, cx, cy, cz};
+  for (int a = 0; a < 4; ++a) {
+    if (!src[a]) continue;
+    CU(cudaMalloc(&c->d_coef[a], sizeof(double) * n + kCbPadBytes));
+    CU(cudaMemcpyAsync(c->d_coef[a], src[a], sizeof(double) * n, cudaMemcpyHostToDevice, c->stream));
+  }
+  CU(cudaStreamSynchronize(c->stream));      // (pageable host arrays)
+  c->vsten = VarStencilOp{(int)nx, (int)ny, (int)nz, n, c->d_coef[0], c->d_coef[1], c->d_coef[2], c->d_coef[3]};
+  // the coefficient planes of the TMA pass: encoded once here (false for odd nx: the generic kernel runs)
+  c->coef_tmap_ok = true;
+  for (int a = 1; a < 4; ++a)
+    if (c->d_coef[a]) c->coef_tmap_ok = c->coef_tmap_ok && tma_encode_dims(c->d_coef[a], nx, ny, nz, &c->coef_tmap[a - 1]);
+  c->nnz = 0;
+  c->op_kind = 3;
+  return CGX_OK;
+}
+
 extern "C" int cgx_set_jacobi_host(cgx_ctx* c, const double* dinv, int64_t n) {
   if (!c) return fail(CGX_ERR_ARG, "cgx_set_jacobi_host: ctx is NULL");
   CU(cudaSetDevice(c->device));
@@ -485,8 +534,8 @@ bool tma_encode_dims(double* ptr, i64 nx, i64 ny, i64 nz, CUtensorMap* out) {
 }
 
 static bool tma_prepare_geom(cgx_ctx* c) {
-  if (c->op_kind != 2 || c->no_tma) return false;
-  const StencilOp& S = c->sten;
+  if ((c->op_kind != 2 && c->op_kind != 3) || c->no_tma) return false;
+  const StencilOp S = c->op_kind == 3 ? StencilOp{c->vsten.nx, c->vsten.ny, c->vsten.nz, 0.0, 0.0, c->vsten.n, 0, 0} : c->sten;
   if (S.nx % 2 != 0 || S.nx < 2) return false;         // TMA needs 16-byte global strides
   if (S.ny < 4 && S.nz > 1) return false;              // 2-D grid viewed as nx x 1 x ny slabs: tiles would idle
   if (!get_encode_tiled()) return false;
@@ -522,9 +571,10 @@ static int setup_tma(cgx_ctx* c, unsigned need) {
   c->halo_ll = false;
   for (auto& ok : c->tmap_ok) ok = false;
   if (!tma_prepare_geom(c)) return CGX_OK;
-  const StencilOp& S = c->sten;
+  const int nx = c->op_kind == 3 ? c->vsten.nx : c->sten.nx, ny = c->op_kind == 3 ? c->vsten.ny : c->sten.ny,
+            nz = c->op_kind == 3 ? c->vsten.nz : c->sten.nz;
   for (int i = 0; i < V_COUNT; ++i)
-    if ((need & (1u << i)) && c->vec[i]) c->tmap_ok[i] = tma_encode_dims(c->vec[i], S.nx, S.ny, S.nz, &c->tmap[i]);
+    if ((need & (1u << i)) && c->vec[i]) c->tmap_ok[i] = tma_encode_dims(c->vec[i], nx, ny, nz, &c->tmap[i]);
   // every fused SpMV pass of the variant must take the TMA kernel for the LL ghost planes
   bool all_ok = true;
   for (int i = 0; i < V_COUNT; ++i)
@@ -558,6 +608,9 @@ void launch_instrument(cgx_ctx* c, Args g) {
     if (c->op_kind == 1) {
       if (c->has_xtrue) instrument_kernel<CsrOp, true><<<grid, kBlock, 0, c->stream>>>(c->csr, g, xin, xtin);
       else instrument_kernel<CsrOp, false><<<grid, kBlock, 0, c->stream>>>(c->csr, g, xin, xtin);
+    } else if (c->op_kind == 3) {
+      if (c->has_xtrue) instrument_kernel<VarStencilOp, true><<<grid, kBlock, 0, c->stream>>>(c->vsten, g, xin, xtin);
+      else instrument_kernel<VarStencilOp, false><<<grid, kBlock, 0, c->stream>>>(c->vsten, g, xin, xtin);
     } else {
       if (c->has_xtrue) instrument_kernel<StencilOp, true><<<grid, kBlock, 0, c->stream>>>(c->sten, g, xin, xtin);
       else instrument_kernel<StencilOp, false><<<grid, kBlock, 0, c->stream>>>(c->sten, g, xin, xtin);
@@ -837,6 +890,11 @@ static int pers_launch(cgx_ctx** cs, int count, const PersGeom& G, int k0, int k
     if (c->pm == 2) return cgx_pers_launch_csr_pm2(cs, count, G, k0, k1);
     if (c->pm == 1) return cgx_pers_launch_csr_pm1(cs, count, G, k0, k1);
     return cgx_pers_launch_csr_pm0(cs, count, G, k0, k1);
+  }
+  if (c->op_kind == 3) {
+    if (c->pm == 2) return cgx_pers_launch_var_pm2(cs, count, G, k0, k1);
+    if (c->pm == 1) return cgx_pers_launch_var_pm1(cs, count, G, k0, k1);
+    return cgx_pers_launch_var_pm0(cs, count, G, k0, k1);
   }
   if (c->pm == 2) return cgx_pers_launch_sten_pm2(cs, count, G, k0, k1);
   if (c->pm == 1) return cgx_pers_launch_sten_pm1(cs, count, G, k0, k1);
@@ -1255,6 +1313,7 @@ static int batch_run(cgx_ctx** cs, int count, const int* variants, const int* ma
       if (cs[j] == c) return fail(CGX_ERR_ARG, "cgx_batch_run: entries %d and %d are the same context", j, i);
     if (c->device != cs[0]->device) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entries on different devices");
     if (c->dist.world > 1) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d is a rank of a partition", i);
+    if (c->op_kind == 3) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d has a variable-coefficient stencil", i);
     if (c->op_kind != cs[0]->op_kind) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: CSR and stencil operators mixed");
     if (c->pm != cs[0]->pm) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: preconditioner modes mixed (%d, %d)", cs[0]->pm, c->pm);
     if (c->capture_req) return fail(CGX_ERR_UNSUPPORTED, "cgx_batch_run: entry %d has a capture set (stream path only)", i);
@@ -1705,6 +1764,11 @@ extern "C" int cgx_spmv_host(cgx_ctx* c, const double* v, double* y, int64_t n) 
     G.nchunk = std::max(1, std::min(cap / std::max(1, ncols), G.nz / std::max(1, c->tma_min_planes)));
     stencil_tma_kernel<SP_PIPE_N, 0, false><<<(int)std::min<i64>((i64)ncols * G.nchunk, cap), kSThreads, tma_smem_bytes(1), c->stream>>>(
         tm, tm, G, g);
+    c->launches++;
+  } else if (c->op_kind == 3 && c->coef_tmap_ok && tma_prepare_geom(c) &&
+             tma_encode_dims(dv, c->vsten.nx, c->vsten.ny, c->vsten.nz, &tm)) {
+    g.u = dy;                          // (the same plainest mode of the variable-coefficient pass)
+    launch_varstencil_tma<SP_PIPE_N, 0, false>(c, g, tm, tm);
     c->launches++;
   } else {
     launch_spmv<SP_PLAIN, 0, false>(c, g, dv, dy);

@@ -23,6 +23,7 @@
 #include "cgx_stencil_tma.cuh"
 #include "cgx_csr_bulk.cuh"
 #include "cgx_persistent.cuh"
+#include "cgx_varstencil.cuh"
 
 using namespace cgx;
 
@@ -61,9 +62,13 @@ struct cgx_ctx {
   cudaStream_t stream = nullptr;
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   // operator
-  int op_kind = 0;  // 0 none, 1 csr, 2 stencil
+  int op_kind = 0;  // 0 none, 1 csr, 2 stencil, 3 variable-coefficient stencil
   CsrOp csr{};
   StencilOp sten{};
+  VarStencilOp vsten{};
+  double* d_coef[4] = {};          // op_kind 3: diag, cx, cy, cz (cz null in 2-D)
+  CUtensorMap coef_tmap[3];        // op_kind 3: cx, cy, cz (encoded by cgx_set_stencil_coef_host)
+  bool coef_tmap_ok = false;
   int* d_ptr = nullptr;
   int* d_idx = nullptr;
   double* d_val = nullptr;
@@ -285,10 +290,12 @@ void cgx_iter_stage_pm2(cgx_ctx* c, int s, const Args& g);
 
 struct PersGeom { int T, nb, R, nslot, slab_cap; unsigned vmask; size_t smem; bool ok; };
 
-// persistent path, per operator kind (cgx_pers.cu compiled with -DCGX_PERS_OP=1 CSR | 2 stencil and -DCGX_PERS_PM=0|1|2)
+// persistent path, per operator kind (cgx_pers.cu compiled with -DCGX_PERS_OP=1 CSR | 2 stencil | 3 variable-coefficient
+// stencil and -DCGX_PERS_PM=0|1|2)
 #define CGX_PERS_DECL(name) int name(cgx_ctx** cs, int count, const PersGeom& G, int k0, int k1)
 CGX_PERS_DECL(cgx_pers_launch_csr_pm0); CGX_PERS_DECL(cgx_pers_launch_csr_pm1); CGX_PERS_DECL(cgx_pers_launch_csr_pm2);
 CGX_PERS_DECL(cgx_pers_launch_sten_pm0); CGX_PERS_DECL(cgx_pers_launch_sten_pm1); CGX_PERS_DECL(cgx_pers_launch_sten_pm2);
+CGX_PERS_DECL(cgx_pers_launch_var_pm0); CGX_PERS_DECL(cgx_pers_launch_var_pm1); CGX_PERS_DECL(cgx_pers_launch_var_pm2);
 // batch of independent solves in one cooperative launch (cgx_batch_run); launch = false: co-residency check only
 #define CGX_PERS_BATCH_DECL(name) int name(cgx_ctx** cs, int count, const int* variants, const PersGeom* G, const int* k1, bool launch)
 CGX_PERS_BATCH_DECL(cgx_pers_batch_csr_pm0); CGX_PERS_BATCH_DECL(cgx_pers_batch_csr_pm1); CGX_PERS_BATCH_DECL(cgx_pers_batch_csr_pm2);

@@ -33,6 +33,23 @@ static void launch_csr_bulk(cgx_ctx* c, const Args& g, const VecIn& in0, const V
                                                                             g, in0, in1, vout);
 }
 
+// TMA-staged pass of the variable-coefficient stencil (cgx_varstencil.cuh): one resident wave of
+// (column, z-chunk) work units, as for stencil_tma_kernel.  tm0 / tm1: the vector(s) the pass reads.
+template <int MODE, int PM, bool MEUR>
+static void launch_varstencil_tma(cgx_ctx* c, Args g, const CUtensorMap& tm0, const CUtensorMap& tm1) {
+  constexpr int nv = NV_OF(MODE);
+  const size_t sm = varstencil_smem_bytes(nv);
+  const int per_sm = ctx_occupancy(c, (const void*)varstencil_tma_kernel<MODE, PM, MEUR>, kSThreads, sm);
+  TmaGeom G = c->geom;
+  const int cap = per_sm * c->sm_count, ncols = G.ntx * G.nty;
+  G.nchunk = std::max(1, std::min(cap / std::max(1, ncols), G.nz / std::max(1, c->tma_min_planes)));
+  const int grid = (int)std::min<i64>((i64)ncols * G.nchunk, cap);
+  // (2-D: no cz map; the kernel never reads its third coefficient map then)
+  const CUtensorMap& tcz = c->vsten.cz ? c->coef_tmap[2] : c->coef_tmap[0];
+  launch_k(varstencil_tma_kernel<MODE, PM, MEUR>, grid, kSThreads, sm, c->stream, use_pdl(c),
+           tm0, tm1, c->coef_tmap[0], c->coef_tmap[1], tcz, c->vsten, G, g);
+}
+
 // Fused SpMV pass of stage MODE (vin/vout only for SP_PLAIN / SP_RESID).
 template <int MODE, int PM, bool MEUR>
 static void launch_spmv(cgx_ctx* c, Args g, const double* vin, double* vout) {
@@ -59,6 +76,11 @@ static void launch_spmv(cgx_ctx* c, Args g, const double* vin, double* vout) {
         launch_k(stencil_tma_kernel<MODE, PM, MEUR>, tgrid, kSThreads, tma_smem_bytes(nv), c->stream, use_pdl(c),
                  c->tmap[v0], c->tmap[v1 < 0 ? v0 : v1], G, g);
         done = true;
+      } else if constexpr (MODE != SP_CG_E && MODE != SP_GV_E) {
+        if (c->op_kind == 3 && c->use_tma && c->coef_tmap_ok && c->tmap_ok[v0] && (v1 < 0 || c->tmap_ok[v1 < 0 ? 0 : v1])) {
+          launch_varstencil_tma<MODE, PM, MEUR>(c, g, c->tmap[v0], c->tmap[v1 < 0 ? v0 : v1]);
+          done = true;
+        }
       }
     }
     if (!done) {
@@ -84,6 +106,8 @@ static void launch_spmv(cgx_ctx* c, Args g, const double* vin, double* vout) {
         } else {
           spmv_kernel<CsrOp, MODE, PM, MEUR><<<grid_for(c, c->n), kBlock, 0, c->stream>>>(c->csr, g, in0, in1, vout);
         }
+      } else if (c->op_kind == 3) {
+        spmv_kernel<VarStencilOp, MODE, PM, MEUR><<<grid_for(c, c->n), kBlock, 0, c->stream>>>(c->vsten, g, in0, in1, vout);
       } else {
         spmv_kernel<StencilOp, MODE, PM, MEUR><<<grid_for(c, c->n), kBlock, 0, c->stream>>>(c->sten, g, in0, in1, vout);
       }

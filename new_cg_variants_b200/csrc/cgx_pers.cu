@@ -1,16 +1,18 @@
 // cgx_pers.cu -- launchers of the persistent cooperative kernels (cgx_persistent.cuh: one variant,
-// or a batch of independent solves) for one operator kind and one preconditioner mode (compiled six times: -DCGX_PERS_OP=1 CSR | 2 matrix-free
-// stencil, -DCGX_PERS_PM=0|1|2).
+// or a batch of independent solves) for one operator kind and one preconditioner mode (compiled nine times: -DCGX_PERS_OP=1 CSR | 2 matrix-free
+// stencil | 3 variable-coefficient stencil (one variant per launch only), -DCGX_PERS_PM=0|1|2).
 #include "cgx_host.h"
 
 #ifndef CGX_PERS_OP
-#error "compile with -DCGX_PERS_OP=1|2"
+#error "compile with -DCGX_PERS_OP=1|2|3"
 #endif
 
 // the kernel's view of context c; its sync counter and PersOut are zeroed on `st`
 template <class Op>
 static int pers_fill_rank(cgx_ctx* c, cudaStream_t st, PersRank<Op>& r) {
-  if constexpr (std::is_same<Op, CsrOp>::value) r.A = c->csr; else r.A = c->sten;
+  if constexpr (std::is_same<Op, CsrOp>::value) r.A = c->csr;
+  else if constexpr (std::is_same<Op, VarStencilOp>::value) r.A = c->vsten;
+  else r.A = c->sten;
   Args g = make_args(c);
   Plan p;                                           // fills scpar / x_true epochs
   plan_apply(c, g, p);
@@ -124,6 +126,10 @@ int CGX_CAT(cgx_pers_launch_csr, _pm, CGX_PERS_PM)(cgx_ctx** cs, int count, cons
 int CGX_CAT(cgx_pers_batch_csr, _pm, CGX_PERS_PM)(cgx_ctx** cs, int count, const int* variants, const PersGeom* G,
                                                   const int* k1, bool launch) {
   return pers_batch_pm<CsrOp, CGX_PERS_PM>(cs, count, variants, G, k1, launch);
+}
+#elif CGX_PERS_OP == 3
+int CGX_CAT(cgx_pers_launch_var, _pm, CGX_PERS_PM)(cgx_ctx** cs, int count, const PersGeom& G, int k0, int k1) {
+  return pers_launch_pm<VarStencilOp, CGX_PERS_PM>(cs, count, G, k0, k1);
 }
 #else
 int CGX_CAT(cgx_pers_launch_sten, _pm, CGX_PERS_PM)(cgx_ctx** cs, int count, const PersGeom& G, int k0, int k1) {

@@ -27,7 +27,7 @@ from pickle import dumps as pickle_dumps, loads as pickle_loads
 import numpy as np
 
 from . import _lib
-from .operators import PoissonStencil
+from .operators import PoissonStencil, VariableStencil
 from .session import _f64
 
 MODES = {"p2p": 1, "nccl": 2}
@@ -36,6 +36,11 @@ MODES = {"p2p": 1, "nccl": 2}
 # ---------------------------------------------------------------------------------------
 # host-side partition logic (pure Python; covered by the CPU tests)
 # ---------------------------------------------------------------------------------------
+def _refuse_variable_stencil(S, who):
+    if isinstance(S, VariableStencil):
+        raise NotImplementedError(f"{who}: a VariableStencil runs on one GPU (Session); partitions are not supported")
+
+
 def slab_grid(S: PoissonStencil):
     """(nx, ny, nz) of the 3-D slab view of a stencil operator: a 2-D nx x ny grid is the
     3-D grid nx x 1 x ny (same canonical term order: y-1, x-1, c, x+1, y+1)."""
@@ -254,6 +259,7 @@ class DistSession(_RankBase):
         either the GLOBAL one, held by every rank, or -- with ``row_block=(row0, row1)`` and
         ``n_global`` -- only this rank's rows (shape (row1-row0, n_global), global column indices);
         the ghost lists are then exchanged through torch.distributed."""
+        _refuse_variable_stencil(S, "DistSession")
         import torch.distributed as dist
         self.group = group
         rank = dist.get_rank(group) if rank is None else rank
@@ -388,6 +394,7 @@ class GroupSession:
         pass
 
     def __init__(self, S, world, dinv=None, devices=None, mode="p2p"):
+        _refuse_variable_stencil(S, "GroupSession")
         if mode != "p2p":
             raise NotImplementedError("GroupSession drives the peer-to-peer scalar exchange only")
         self._lib = _lib.load()

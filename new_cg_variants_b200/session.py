@@ -11,7 +11,7 @@ import numpy as np
 import scipy.sparse as sps
 
 from . import _lib
-from .operators import PoissonStencil, canonical_csr
+from .operators import PoissonStencil, VariableStencil, canonical_csr
 
 
 def _f64(a, n=None, name="array"):
@@ -40,6 +40,12 @@ class Session:
             self.n = A.shape[0]
             self.nnz = A.nnz
             _lib.check(self._lib.cgx_set_stencil(self._ctx, A.dim, A.nx, A.ny, A.nz, A.diag, A.off))
+        elif isinstance(A, VariableStencil):
+            self.kind = "varstencil"
+            self.n = A.shape[0]
+            self.nnz = A.nnz
+            _lib.check(self._lib.cgx_set_stencil_coef_host(self._ctx, A.dim, A.nx, A.ny, A.nz, _lib.dptr(A.diag),
+                                                           _lib.dptr(A.cx), _lib.dptr(A.cy), _lib.dptr(A.cz)))
         else:
             A = canonical_csr(A)
             self.kind = "csr"
@@ -291,6 +297,8 @@ def solve_batch(items, histories=_lib.HIST_NAMES, return_x=True, tol=None):
     items = [tuple(it) for it in items]
     if not items:
         raise ValueError("solve_batch: no items")
+    if any(getattr(it[0], "kind", None) == "varstencil" for it in items):
+        raise NotImplementedError("solve_batch: a VariableStencil runs one solve per launch (Session.solve)")
     sessions, xts = [], []
     for it in items:
         if len(it) not in (5, 6):
@@ -332,6 +340,6 @@ def solve_batch(items, histories=_lib.HIST_NAMES, return_x=True, tol=None):
 
 
 def diagonal_of(A):
-    if isinstance(A, PoissonStencil) or sps.issparse(A):
+    if isinstance(A, (PoissonStencil, VariableStencil)) or sps.issparse(A):
         return np.asarray(A.diagonal(), dtype=np.float64)
     return np.asarray(np.diag(A), dtype=np.float64)
